@@ -116,6 +116,29 @@ class ClockSampler:
                 "reasons": sorted(reasons), "samples": len(sm)}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, arrays: dict, rank: int, world: int) -> None:
+    """Write each array as <out_dir>/<name>.npy (<out_dir>/rank<r>/ when several ranks run): float64 stays float64, every
+    other dtype becomes float32 (the integer outputs are far below 2^24, so exactly).  When the whole set exceeds 64 MB, every
+    array keeps the same fixed, seeded sample of frames (first axis), and sample_index.npy holds their indices."""
+    host = {k: v.cpu().numpy() for k, v in arrays.items()}
+    host = {k: v if v.dtype == np.float64 else v.astype(np.float32) for k, v in host.items()}
+    n = len(next(iter(host.values())))
+    per_frame = sum(v.nbytes for v in host.values()) / max(n, 1)
+    budget = DUMP_LIMIT_BYTES - (64 << 10)                        # room for the .npy headers
+    if n * per_frame > budget:
+        keep = int(budget // (per_frame + 8))
+        idx = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        host = {k: v[idx] for k, v in host.items()}
+        host["sample_index"] = idx.astype(np.float64)
+    d = Path(out_dir) / (f"rank{rank}" if world > 1 else "")
+    d.mkdir(parents=True, exist_ok=True)
+    for k, v in host.items():
+        np.save(d / f"{k}.npy", v)
+
+
 def make_poses(n: int, seed: int):
     rng = np.random.default_rng(seed)
     truth = np.array([synth.random_pose(rng) for _ in range(n)])
@@ -308,6 +331,9 @@ def run_gpu(args):
         dist.barrier()
     launches = ctx.launch_count() - l0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        # what a caller of the refinement receives for the batch of the last timed step
+        dump_outputs(args.dump_outputs, {k: res[k] for k in ("pose", "cost", "n_valid", "evals", "status", "left_roi")}, rank, world)
     gather_ok = True
     if world > 1:
         # every rank holds every rank's poses: its own block is bit-identical, and all ranks agree on a checksum of the whole
@@ -973,7 +999,14 @@ def main():
     ap.add_argument("--stream-input", default="detections", choices=["detections", "pixels"],
                     help="streams workload: tag detections handed in (BASELINE config 5), or frames only - the detector runs on the device")
     ap.add_argument("--no-streams", action="store_true", help="skip the config-3/4/5 legs of the default line")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="default workload: write the refinement outputs of the last timed step to DIR/<name>.npy (float32/float64), "
+                         "to compare two builds on the same seeded inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "dpr"):
+        ap.error("--dump-outputs applies to the default workload (--workload dpr) of this implementation")
     if args.frames is None:
         args.frames = 8192 if args.workload == "lk" else 4096
     ensure_library()

@@ -6,8 +6,8 @@ reference`` legs of ``bench.py`` import it, and only as the checker.
 
 Parity status per stage (see DESIGN.md):
   * APE (detect_pose.py:467-574 + cv2.solvePnP): pinned - ``ape_oracle`` is
-    checked against the unmodified reference imported from /root/reference
-    (``ref_runner``) and against committed golden vectors generated by it.
+    checked against committed golden vectors that the unmodified reference
+    generated (``make_golden`` driving it through ``ref_runner``).
   * pyramid / LK: the reference snapshot has no such code; the frozen spec is
     OpenCV 4.13 ``pyrDown`` / ``Scharr`` / ``calcOpticalFlowPyrLK`` (binary in
     this image, third-party, source absent).  ``lk_oracle`` calls it and also

@@ -30,7 +30,9 @@ def test_library_exports_every_declared_symbol(lib_built):
 
 
 def test_library_is_sm100a_only(lib_built):
-    out = subprocess.run(["cuobjdump", "--list-elf", str(lib_built)], capture_output=True, text=True)
+    from accurate_aprilgroup_tracking_b200 import _build
+    cuobjdump = Path(_build._nvcc()).with_name("cuobjdump")       # the toolkit that built the library, on PATH or not
+    out = subprocess.run([str(cuobjdump), "--list-elf", str(lib_built)], capture_output=True, text=True)
     if out.returncode != 0:
         pytest.skip("cuobjdump unavailable")
     archs = set(re.findall(r"sm_\d+a?", out.stdout))

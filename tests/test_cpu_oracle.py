@@ -3,7 +3,7 @@ import numpy as np
 import pytest
 
 from accurate_aprilgroup_tracking_b200 import synth
-from oracle import ape_oracle, dpr_oracle, lk_oracle, make_golden, ref_runner
+from oracle import ape_oracle, dpr_oracle, lk_oracle, make_golden
 from tests import util
 
 GOLDEN = make_golden.GOLDEN
@@ -39,40 +39,6 @@ def test_ape_oracle_reproduces_reference_golden_bit_exact():
 def test_object_points_match_reference_golden():
     g = np.load(GOLDEN / "ape_sequence.npz")
     assert np.allclose(synth.object_points(), g["all_objpts"], atol=1e-9)
-
-
-@pytest.mark.skipif(not ref_runner.reference_available(), reason="/root/reference not mounted")
-def test_ape_oracle_matches_live_reference():
-    cam = synth.CAMERA_VGA
-    rr = ref_runner.ReferenceRunner(cam.mtx, None, True)
-    orc = ape_oracle.ApeOracle(ape_oracle.group_from_json(synth.april_group_dict()), cam.mtx, None, True)
-    traj = synth.trajectory(1234, 40)
-    rng = np.random.default_rng(1234)
-    for f in range(40):
-        dets = synth.detections(traj[f], cam, rng)
-        if f == 15:
-            dets = []
-        a = rr.estimate(dets)
-        orc.step(dets)
-        b = orc.snapshot()
-        for key in ("prev", "guess"):
-            assert (a[key] is None) == (b[key] is None)
-            if a[key] is not None:
-                assert np.array_equal(np.concatenate(a[key]), np.concatenate(b[key]))
-
-
-@pytest.mark.skipif(not ref_runner.reference_available(), reason="/root/reference not mounted")
-def test_reference_detect_and_get_pose_runs_with_stub():
-    cam = synth.CAMERA_VGA
-    rr = ref_runner.ReferenceRunner(cam.mtx, None, True)
-    rng = np.random.default_rng(3)
-    pose = synth.trajectory(9, 2)[0]
-    dets = synth.detections(pose, cam, rng)
-    frame = np.repeat(synth.render(pose, cam, 1)[:, :, None], 3, axis=2)
-    snap = rr.detect_and_get_pose(frame, dets, margins=[100.0] * (len(dets) - 1) + [10.0])   # last one filtered out
-    assert snap["prev"] is not None
-    dr, dt = util.pose_diff(np.concatenate(snap["prev"]), pose)
-    assert dr < 0.02 and dt < 2e-3
 
 
 def test_decision_margin_filter():
