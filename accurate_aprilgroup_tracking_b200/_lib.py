@@ -10,10 +10,7 @@ from __future__ import annotations
 import ctypes as C
 from pathlib import Path
 
-import os
-
-# AGT_LIBRARY: another build of the same ABI (A/B measurements of kernel variants; scripts/ only)
-LIB_PATH = Path(os.environ["AGT_LIBRARY"]) if os.environ.get("AGT_LIBRARY") else Path(__file__).resolve().parent / "csrc" / "libagt.so"
+LIB_PATH = Path(__file__).resolve().parent / "csrc" / "libagt.so"
 
 AGT_MAX_LEVELS = 4
 AGT_MAX_TAGS = 16

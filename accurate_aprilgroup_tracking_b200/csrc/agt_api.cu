@@ -114,22 +114,11 @@ extern "C" int agt_create(int device, agt_ctx** out) {
   ctx->stream = ctx->own_stream;
   ctx->roi_upload = 1;
   {
-    // whole-frame pyramids in one pass over HBM: measured slower than the per-level launches (2.75 against 2.46 ms per 4096
-    // frames: the HBM traffic drops to the algorithmic 2.8 MB per frame, but half of the CTA's warps follow the other half and
-    // the kernel is issue-bound), so it is opt-in: AGT_K1_FUSED=1 (scripts/k1_fused_probe.py)
-    const char* e = getenv("AGT_K1_FUSED");
-    ctx->k1_fused = e && e[0] == '1';
-  }
-  {
     // LK of a small batch (a frame-step of the stream pipeline) is a wait for the slowest corner: a warp per pyramid level
     // (lk_levels_kernel) halves that latency; large batches are throughput-bound and keep one warp per corner.  A machine-full
     // of corners in the level-parallel layout = 4 x 8 CTAs of four warps per SM.
     const char* e = getenv("AGT_LK_SPLIT_MAX");
     ctx->lk_split_max = e ? atoi(e) : 8 * ctx->sm_count;
-  }
-  {
-    const char* e = getenv("AGT_TAG_SEPARATE_PASSES");
-    ctx->tag_separate_passes = e ? atoi(e) : 0;
   }
   {
     unsigned hc = std::thread::hardware_concurrency();

@@ -47,8 +47,6 @@ struct agt_ctx {
   short* d_remap_tab;            // [1024][4] int16 bilinear weights of cv::remap (device)
   agt_model model;
   int64_t launches;
-  int k1_fused;                  // whole-frame pyramids in one pass (pyr_fused_kernel); AGT_K1_FUSED=0 selects the per-level launches
-  int k1_fused_per_sm;           // resident CTAs per SM of that kernel (0: not asked yet)
   int lk_split_max;              // agt_lk of at most this many corners runs a warp per pyramid level (AGT_LK_SPLIT_MAX; 0: never)
   int roi_upload;                // agt_refine_host uploads only the rectangle a refinement can read
   int64_t last_h2d_bytes;        // host->device bytes of the last agt_refine_host call
@@ -69,7 +67,6 @@ struct agt_ctx {
   uint64_t* d_tag_codes;         // tag family (36-bit code words) of agt_decode_tags / agt_detect_tags
   int n_tag_codes;
   int tag_threshold;             // agt_set_tag_threshold: 0 auto, 1 one threshold per search window, 2 local white level
-  int tag_separate_passes;       // AGT_TAG_SEPARATE_PASSES=1: the quadrilateral passes as launches of their own even for batches (A/B)
   // scratch device memory owned by the context (host entry points)
   void* scratch[8];
   size_t scratch_bytes[8];

@@ -30,10 +30,7 @@ namespace cg = cooperative_groups;
 
 namespace {
 
-#ifndef AGT_DPR_THREADS
-#define AGT_DPR_THREADS 256      // (A/B builds: scripts/build_variant.py -DAGT_DPR_THREADS=...)
-#endif
-constexpr int DPR_THREADS = AGT_DPR_THREADS;
+constexpr int DPR_THREADS = 256;
 constexpr int DPR_WARPS = DPR_THREADS / 32;
 constexpr int TILE_ROWS = AGT_DPR_TILE_ROWS;
 constexpr int TILE_PITCH = AGT_DPR_TILE_PITCH;

@@ -7,11 +7,7 @@
 #pragma once
 #include "agt_common.cuh"
 
-#ifndef AGT_DPR_TILE_ROWS_OVERRIDE
 constexpr int AGT_DPR_TILE_ROWS = 270;
-#else
-constexpr int AGT_DPR_TILE_ROWS = AGT_DPR_TILE_ROWS_OVERRIDE;
-#endif
 constexpr int AGT_DPR_TILE_PITCH = 288;          // 272 + 16 B alignment slack; 2 CTAs of 76.5 KB per SM
 constexpr int AGT_DPR_DRIFT_MARGIN = 8;          // level pixels the projection may drift during LM
 

@@ -114,21 +114,6 @@ __device__ __forceinline__ float reduce_lanes4(float acc) {
 // (profiles/r01_lk_variants.log).
 __device__ __forceinline__ long long warp_sum_wide(int v) { return agt_warp_sum((long long)v); }
 
-#ifdef AGT_LK_DEBUG
-// debug build only (scripts/lk_debug_probe.py): per-level / per-iteration sums of one corner
-__device__ float g_lk_dbg[8192];
-__device__ int g_lk_dbg_gid = -1, g_lk_dbg_n = 0;
-#define LK_DBG(...)                                                                     \
-  do {                                                                                  \
-    if (gid == g_lk_dbg_gid && lane == 0) {                                             \
-      const float v_[] = {__VA_ARGS__};                                                 \
-      for (unsigned q_ = 0; q_ < sizeof(v_) / 4; ++q_) if (g_lk_dbg_n < 8192) g_lk_dbg[g_lk_dbg_n++] = v_[q_]; \
-    }                                                                                   \
-  } while (0)
-#else
-#define LK_DBG(...) do {} while (0)
-#endif
-
 struct Weights { int w00, w01, w10, w11; };
 
 __device__ __forceinline__ Weights make_weights(float a, float b) {
@@ -506,7 +491,6 @@ __device__ __forceinline__ void lk_corner(WarpSmem& S, const int lane, const int
     float A11 = __fmul_rn(__fadd_rn(__shfl_sync(0xffffffffu, acc, 4), A11s), FLT_SCALE);
     float A12 = __fmul_rn(__fadd_rn(__shfl_sync(0xffffffffu, acc, 5), A12s), FLT_SCALE);
     float A22 = __fmul_rn(__fadd_rn(__shfl_sync(0xffffffffu, acc, 6), A22s), FLT_SCALE);
-    LK_DBG(-1.f, (float)level, A11, A12, A22, px, py);
     float D = __fsub_rn(__fmul_rn(A11, A22), __fmul_rn(A12, A12));
     float dif = __fsub_rn(A11, A22);
     float disc = __fadd_rn(__fmul_rn(dif, dif), __fmul_rn(__fmul_rn(4.f, A12), A12));
@@ -615,7 +599,6 @@ __device__ __forceinline__ void lk_corner(WarpSmem& S, const int lane, const int
       const float ib1 = __fadd_rn(__shfl_sync(0xffffffffu, ch, 8), __shfl_sync(0xffffffffu, lanes4, 0));
       const float ib2 = __fadd_rn(__shfl_sync(0xffffffffu, ch, 9), __shfl_sync(0xffffffffu, lanes4, 4));
       __syncwarp();
-      LK_DBG((float)j, ib1, ib2, nx, ny);
       float b1 = __fmul_rn(ib1, FLT_SCALE);
       float b2 = __fmul_rn(ib2, FLT_SCALE);
       float dx = __fmul_rn(__fsub_rn(__fmul_rn(A12, b2), __fmul_rn(A22, b1)), D);
@@ -796,22 +779,6 @@ __global__ void lk_merge_kernel(const float* __restrict__ tracked, const uint8_t
 }
 
 }  // namespace
-
-#ifdef AGT_LK_DEBUG
-extern "C" int agt_lk_debug_set(int gid) {
-  int zero = 0;
-  cudaMemcpyToSymbol(g_lk_dbg_gid, &gid, sizeof(int));
-  return (int)cudaMemcpyToSymbol(g_lk_dbg_n, &zero, sizeof(int));
-}
-extern "C" int agt_lk_debug_get(float* host, int cap) {
-  int n = 0;
-  cudaDeviceSynchronize();
-  cudaMemcpyFromSymbol(&n, g_lk_dbg_n, sizeof(int));
-  if (n > cap) n = cap;
-  cudaMemcpyFromSymbol(host, g_lk_dbg, sizeof(float) * n);
-  return n;
-}
-#endif
 
 extern "C" int agt_lk_merge(agt_ctx* ctx, const float* d_tracked_pts, const uint8_t* d_status, const uint8_t* d_prev_valid,
                             float* d_img_pts, uint8_t* d_valid, int32_t* d_n_tags, int32_t* d_tracked_tags, int batch, int n_pts) {

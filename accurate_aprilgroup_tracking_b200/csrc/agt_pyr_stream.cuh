@@ -53,20 +53,13 @@ __device__ __forceinline__ void cp_async4(uint32_t smem, const void* gmem, int s
   asm volatile("{ .reg .pred p; setp.ne.s32 p, %2, 0; @p cp.async.ca.shared.global [%0], [%1], 4; }" ::"r"(smem), "l"(gmem), "r"(size));
 }
 
-// Hooks of the strip routine for callers that chain levels inside one kernel (pyr_fused_kernel): wait_row(r) runs before source
-// row r is requested, rows_done(n) after output rows < n of the strip's destination have been stored.  The default does nothing.
-struct PyrNoSync {
-  __device__ __forceinline__ void wait_row(int) const {}
-  __device__ __forceinline__ void rows_done(int) const {}
-};
-
 // One warp computes output rows [oy0, oy1) x the 8*NW output columns of each lane starting at ox0 (ix0 = 2*ox0 in the
 // source, whose width w is a multiple of 16 and whose rows are 16 B aligned); columns >= xo1 (a multiple of 8) are not
 // stored.  ring0 = shared-memory address of this warp's ring of (PF_Q + 4) rows of (16 + 16*NW*32 + 16) bytes.
-template <int PF_Q, int NW, class Sync = PyrNoSync>
+template <int PF_Q, int NW>
 __device__ __forceinline__ void agt_pyr_down_strip(const uint8_t* __restrict__ img, int w, int h, int64_t spitch,
                                                    uint8_t* __restrict__ out, int64_t dpitch, int ox0, int xo1, int oy0, int oy1,
-                                                   int lane, uint32_t ring0, const Sync sync = Sync()) {
+                                                   int lane, uint32_t ring0) {
   constexpr int NWORD = 4 * NW;                // own 32-bit words per lane and row
   constexpr int RPITCH = 16 + 16 * NW * 32 + 16;
   constexpr int PF_RING = PF_Q + 4;
@@ -84,7 +77,6 @@ __device__ __forceinline__ void agt_pyr_down_strip(const uint8_t* __restrict__ i
     int rr = h - 1 - abs(h - 1 - abs(r_next));
     const uint8_t* row = img + (int64_t)rr * spitch;
     const bool live = issued < n_in;
-    if (live) sync.wait_row(rr);
 #pragma unroll
     for (int k = 0; k < NW; ++k) cp_async16(req_slot + lane_main + 16 * k, row + ix0 + 16 * k, live ? plan.unit_size[k] : 0);
     cp_async4(req_slot + plan.refl_dst, row + w - 4, live ? plan.refl_size : 0);
@@ -136,7 +128,6 @@ __device__ __forceinline__ void agt_pyr_down_strip(const uint8_t* __restrict__ i
     } else {
       if (ox0 < xo1) *reinterpret_cast<uint2*>(o) = make_uint2(px[0], px[1]);      // xo1 % 8 == 0 on this path
     }
-    sync.rows_done(oy + 1);
   };
 
 #pragma unroll

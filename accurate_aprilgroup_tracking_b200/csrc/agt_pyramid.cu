@@ -250,87 +250,6 @@ pyr_roi_chain_kernel(agt_pyramid pyr, const int32_t* __restrict__ rects, int rec
   }
 }
 
-// Whole-frame pyramid in ONE pass over HBM: a CTA takes whole frames; two producer warps stream level 0 into level 1 (one
-// column block of 512 pixels each, top to bottom without a break), a third warp follows them from level 1 to level 2 and a
-// fourth from level 2 to level 3.  The followers request a source row as soon as the warps above have stored it - a few rows
-// behind, i.e. out of the L2 cache - so levels 1 and 2 cross the HBM interface once (written), where the per-level launches read
-// them back (3.40 MB of traffic per 1080p frame against 2.754 MB algorithmic).  No CTA barrier: each warp publishes the number
-// of rows it has stored in shared memory (fence, then the count; counts only grow, frames are handed out statically as
-// frame = blockIdx.x + k gridDim.x, so producers may run ahead into their next frame), a follower spins on the counts of the
-// warps above before it requests a row.  Every warp runs the SAME code - one call site of the 16-pixels-per-lane strip routine
-// with the warp's own level and column block (a first version with one inlined copy of the routine per role spent four of five
-// issue slots waiting for instruction fetch, and with strips of 32 rows between hand-overs 145 MB of level 0 went through the
-// L2 between the store and the load of a row, which therefore came back from HBM: profiles/r02_ncu_k1_fused_first.txt).
-// Same streaming warp routine, same bits as the per-level kernels.
-#ifndef AGT_K1_FUSED_Q
-#define AGT_K1_FUSED_Q 6
-#endif
-#ifndef AGT_K1_FUSED_SLEEP
-#define AGT_K1_FUSED_SLEEP 400
-#endif
-#ifndef AGT_K1_FUSED_CTAS
-#define AGT_K1_FUSED_CTAS 4
-#endif
-template <int Q>
-struct FusedCfg {
-  static constexpr int P = 2;                           // producer warps = column blocks of level 1 (16 pixels per lane: 512 per warp)
-  static constexpr int WARPS = P + 2;
-  static constexpr int RPITCH2 = 16 + 16 * 2 * 32 + 16;
-  static constexpr int RING = (Q + 4) * RPITCH2;
-  static constexpr int SMEM = WARPS * RING + 64;
-};
-
-struct FusedSync {
-  volatile int* prog;        // rows stored per warp, all frames so far
-  int wid, lane;
-  int n_above, first_above;  // the warps whose output this warp reads
-  int base_src, base_dst;    // rows of the frames before the current one (source level / own level)
-  __device__ __forceinline__ void wait_row(int r) const {
-    if (n_above == 0) return;
-    const int need = base_src + r + 1;
-    // (a follower is several times faster than the warps it follows: it sleeps about as long as they need for a row)
-    while (prog[first_above] < need || prog[first_above + n_above - 1] < need) __nanosleep(AGT_K1_FUSED_SLEEP);
-    __threadfence_block();                               // acquire: the row announced by the count is what the copy reads
-  }
-  __device__ __forceinline__ void rows_done(int n) const {
-    __threadfence_block();                               // release: every lane's stores of the row before the count
-    __syncwarp();
-    if (lane == 0) prog[wid] = base_dst + n;
-  }
-};
-
-template <int Q>
-__global__ void __launch_bounds__(FusedCfg<Q>::WARPS * 32, AGT_K1_FUSED_CTAS)
-pyr_fused_kernel(agt_pyramid pyr, int batch) {
-  using Cfg = FusedCfg<Q>;
-  extern __shared__ __align__(16) uint8_t s_dyn[];
-  volatile int* s_prog = reinterpret_cast<volatile int*>(s_dyn);
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  if (threadIdx.x < 16) s_prog[threadIdx.x] = 0;
-  __syncthreads();
-  const uint32_t ring0 = (uint32_t)__cvta_generic_to_shared(s_dyn) + 64 + wid * Cfg::RING;
-  // role of this warp: the level it writes and its column block
-  const int l = wid < Cfg::P ? 1 : (wid == Cfg::P ? 2 : 3);
-  const int cb = l == 1 ? wid : 0;
-  const int sw = pyr.width[l - 1], shh = pyr.height[l - 1], ow = pyr.width[l], oh = pyr.height[l];
-  const bool live = cb * 512 < ow;
-  const int64_t spitch = pyr.pitch[l - 1], dpitch = pyr.pitch[l], sstride = pyr.frame_stride[l - 1], dstride = pyr.frame_stride[l];
-  const uint8_t* src = pyr.data[l - 1];
-  uint8_t* dst = pyr.data[l];
-  FusedSync sync;
-  sync.prog = s_prog; sync.wid = wid; sync.lane = lane;
-  sync.n_above = l == 1 ? 0 : (l == 2 ? Cfg::P : 1);
-  sync.first_above = l == 2 ? 0 : Cfg::P;
-  sync.base_src = 0; sync.base_dst = 0;
-  for (int frame = blockIdx.x; frame < batch; frame += gridDim.x) {
-    if (live)
-      agt_pyr_down_strip<Q, 2, FusedSync>(src + frame * sstride, sw, shh, spitch, dst + frame * dstride, dpitch, cb * 512 + lane * 16, ow, 0, oh,
-                                          lane, ring0, sync);
-    sync.base_src += shh; sync.base_dst += oh;
-    if (!live && lane == 0) s_prog[wid] = sync.base_dst;          // a column block beyond the level's width: nothing to wait for
-  }
-}
-
 // Scharr: one thread per pixel pair; loads go through L1.  Not on the hot path
 // (the LK and refinement kernels derive gradients on the fly from the u8 levels);
 // exported so the derivative planes themselves can be checked bit-exactly.
@@ -492,43 +411,6 @@ static int build_pyramid_impl(agt_ctx* ctx, const agt_pyramid* pyr, int batch, c
       pyr_roi_chain_kernel<6, 8><<<blocks, PF_WARPS * 32, 0, ctx->stream>>>(*pyr, d_rects, rect_stride, batch, wide_mask);
       AGT_LAUNCH_CHECK(ctx);
       return AGT_OK;
-    }
-  }
-  // whole frames, four levels, batches that fill the machine: one pass over HBM (pyr_fused_kernel)
-  if (d_rects == nullptr && d_mask == nullptr && pyr->levels == 4 && batch >= 2 * ctx->sm_count && ctx->k1_fused) {
-    bool ok = pyr->width[1] <= 1024 && pyr->width[2] <= 512 && pyr->width[3] % 8 == 0 && pyr->height[3] >= 4;
-    for (int l = 1; l < 4 && ok; ++l) {
-      const int w = pyr->width[l - 1], h = pyr->height[l - 1];
-      ok = pyr->data[l - 1] && pyr->data[l] && pyr->width[l] == (w + 1) / 2 && pyr->height[l] == (h + 1) / 2 && (w & 15) == 0 && w >= 16 && h >= 4 &&
-           ((reinterpret_cast<uintptr_t>(pyr->data[l - 1]) | (uintptr_t)pyr->pitch[l - 1] | (uintptr_t)pyr->frame_stride[l - 1]) & 15) == 0 &&
-           ((reinterpret_cast<uintptr_t>(pyr->data[l]) | (uintptr_t)pyr->pitch[l] | (uintptr_t)pyr->frame_stride[l]) & 15) == 0 &&
-           pyr->pitch[l - 1] >= w && pyr->pitch[l] >= pyr->width[l];
-    }
-    if (ok) {
-      using Cfg = FusedCfg<AGT_K1_FUSED_Q>;
-      auto kern = pyr_fused_kernel<AGT_K1_FUSED_Q>;
-      static_assert(Cfg::WARPS <= 16, "progress counters");
-      if (ctx->k1_fused_per_sm == 0) {
-        AGT_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM));
-        int n = 0;
-        AGT_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, kern, Cfg::WARPS * 32, Cfg::SMEM));
-        ctx->k1_fused_per_sm = n >= 1 ? n : -1;
-      }
-      const int per_sm = ctx->k1_fused_per_sm;
-      if (per_sm >= 1) {
-        // frames are handed out statically: take the number of resident CTAs per SM that wastes the least of the last wave
-        int best = per_sm;
-        double best_eff = 0.0;
-        for (int c = per_sm; c >= (per_sm + 1) / 2; --c) {
-          const int64_t slots = (int64_t)c * ctx->sm_count, waves = (batch + slots - 1) / slots;
-          const double eff = (double)batch / (double)(waves * slots);
-          if (eff > best_eff + 0.02) { best_eff = eff; best = c; }
-        }
-        const int64_t slots = (int64_t)best * ctx->sm_count;
-        kern<<<(unsigned)(batch < slots ? batch : slots), Cfg::WARPS * 32, Cfg::SMEM, ctx->stream>>>(*pyr, batch);
-        AGT_LAUNCH_CHECK(ctx);
-        return AGT_OK;
-      }
     }
   }
   for (int l = 1; l < pyr->levels; ++l) {

@@ -19,9 +19,7 @@
 // between two float32 positions - and the launch lasts as long as its slowest corner.  With 10 the ids and corners of the probe
 // frames are unchanged (scripts/tag_detect_probe.py) and the pass takes 32 instead of 57 us; cv2.aruco's own refinement stops
 // far earlier (cornerRefinementMinAccuracy 0.1 px).
-#ifndef AGT_TAG_SUBPIX_ITERS
-#define AGT_TAG_SUBPIX_ITERS 10
-#endif
+constexpr int TAG_SUBPIX_ITERS = 10;
 
 namespace {
 
@@ -1105,7 +1103,7 @@ extern "C" int agt_detect_tags_roi(agt_ctx* ctx, const uint8_t* d_gray, int w, i
   comp_stats_kernel<<<grid_ne, 256, 0, st>>>(w, h, d_rects, rect_stride, label, nent, entries, mask_stride, stats, overflow);
   boundary_list_kernel<<<grid_ne, 256, 0, st>>>(w, h, d_rects, rect_stride, label, mask, mask_stride, nent, entries, overflow, run_code, ent_base, stats,
                                                 nlist, far_list);
-  if (batch >= 8 && ctx->tag_separate_passes == 0) {
+  if (batch >= 8) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)batch * FIT_CLUSTER);
     cfg.blockDim = dim3(FIT_THREADS);
@@ -1129,7 +1127,7 @@ extern "C" int agt_detect_tags_roi(agt_ctx* ctx, const uint8_t* d_gray, int w, i
   if (refine_win > 0) {
     // only the corners of emitted quads (the validity flag of a quad, four times), each with its own window
     if ((rc = agt_corner_subpix_windows(ctx, d_gray, w, h, pitch, stride, quads, ws + o_win, ws + o_win, refined, batch, 4 * max_quads,
-                                        refine_win, AGT_TAG_SUBPIX_ITERS, 1e-3)))
+                                        refine_win, TAG_SUBPIX_ITERS, 1e-3)))
       return rc;
     use = refined;
   }

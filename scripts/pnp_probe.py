@@ -1,6 +1,6 @@
 """K3 latency probe (run on the GPU box): one warp per frame, so a 64-frame step is one dependent chain per warp and the launch time is
 the latency of the slowest frame.  Times agt_pnp back to back for a stream-sized batch (64) and for batches that fill the machine.
-    [AGT_LIBRARY=scripts/build/<variant>.so] python scripts/pnp_probe.py"""
+    python scripts/pnp_probe.py"""
 import sys, numpy as np
 sys.path.insert(0, '.')
 import torch
