@@ -526,14 +526,15 @@ class AgtContext:
         res["redo"] = redo
         return res
 
-    def refine_fused(self, pyr: Pyramid, init, n_hyp: int = 1, batch: Optional[int] = None):
+    def refine_fused(self, pyr: Pyramid, init, n_hyp: int = 1, batch: Optional[int] = None, mask=None):
         """Refinement from level 0 alone (K1 fused into K4), exact by construction: every refinement builds the
         region of interest of its own pyramid level inside the kernel; frames whose refinement read outside that
-        region (``left_roi``) get the full pyramid and are refined again, all without leaving the device."""
+        region (``left_roi``) get the full pyramid and are refined again, all without leaving the device.
+        mask [B] u8: frames with 0 are skipped, as in ``refine``."""
         t = self.torch
         b = int(pyr.batch if batch is None else batch)
         ini = self._dev(init, t.float64).reshape(b, n_hyp, 6)
-        res = self.refine(pyr, ini, n_hyp, b, fused=True)
+        res = self.refine(pyr, ini, n_hyp, b, mask=mask, fused=True)
         redo = t.empty(b, dtype=t.uint8, device=self.tdev)
         self._check(self.lib.agt_any_flag(self.h, self._p(res["left_roi"]), n_hyp, self._p(redo), b))
         self.build_pyramid_masked(pyr, redo, b)

@@ -55,7 +55,8 @@ constexpr double TOL_ROT = 5e-6, TOL_TRANS = 1e-6;
 constexpr double AITKEN_COS2 = 0.64, AITKEN_QMAX = 0.75, ALPHA_MIN = 0.25, ALPHA_MAX = 4.0;
 // a trial pose is accepted unless the cost rises by more than this fraction (oracle/dpr_oracle.py: the Scharr gradient is not
 // the exact derivative of the bilinear interpolant, so near convergence the cost moves by ~1e-5 of itself either way; the
-// slack lets the loop contract onto J^T r = 0 instead of stalling where that noise first rejects a step)
+// slack lets the loop contract onto J^T r = 0 instead of stalling where that noise first rejects a step); no trial above the
+// cost at the initial pose is accepted, so that the slack cannot compound into a run that ends worse than it started
 constexpr double ACCEPT_SLACK = 1e-2;
 
 struct DprShared {
@@ -87,6 +88,7 @@ struct DprShared {
   double Pc[12];         // accepted pose: rotation (row-major) + translation
   double Hb[27];         // normal equations at the accepted pose: H (21, packed upper triangle by rows) + b (6)
   double dstep[6], cc, lam;   // dstep: the applied step alpha * d of the pending trial
+  double c0;             // cost at the initial pose: the bound of every accepted cost
   double dgn[6], dprev[6], alpha;   // solve's step of the pending trial / of the last accepted one (Aitken step length)
   int have_prev;
   int nc, evals, status;
@@ -768,7 +770,7 @@ dpr_kernel(agt_pyramid pyr, agt_camera cam, const float4* __restrict__ samples, 
         // |step| against the tolerances, squared on both sides (no square root on the critical path)
         const double* ds = S.dstep;
         const double nw2 = ds[0] * ds[0] + ds[1] * ds[1] + ds[2] * ds[2], nt2 = ds[3] * ds[3] + ds[4] * ds[4] + ds[5] * ds[5];
-        if (nn > 0 && cn < cc * (1.0 + ACCEPT_SLACK)) {
+        if (nn > 0 && cn < cc * (1.0 + ACCEPT_SLACK) && cn <= S.c0) {
           accept = true;
           lam = fmax(lam * 0.1, LAMBDA_MIN);
           if (nw2 < TOL_ROT * TOL_ROT && nt2 < TOL_TRANS * TOL_TRANS) status = AGT_DPR_CONVERGED; else need_step = true;
@@ -845,6 +847,7 @@ dpr_kernel(agt_pyramid pyr, agt_camera cam, const float4* __restrict__ samples, 
         S.alpha = alpha; S.have_prev = have_prev;
         S.stop = need_step ? 0 : 1;
         S.cc = cc; S.lam = lam; S.evals = evals; S.status = status;
+        if (evals == 1) S.c0 = cn;
         if (accept) S.nc = nn;
       }
     }

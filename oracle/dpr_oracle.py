@@ -46,7 +46,8 @@ reduces/solves in float64):
            trial = (exp(alpha d_w) R, t + alpha d_t); one evaluation per trial
            (only while lambda <= lambda0, the undamped regime: a step solved with a larger lambda has alpha = 1 and is not
            remembered as d_prev - steps of different damping are not comparable)
-           accept iff c_trial < c (1 + 1e-2): lambda <- max(lambda/10, 1e-9), d_prev <- d;
+           accept iff c_trial < c (1 + 1e-2) and c_trial <= c_0, the cost at the initial pose:
+           lambda <- max(lambda/10, 1e-9), d_prev <- d;
            else lambda <- 10 lambda, alpha <- 1, d_prev forgotten.
            The slack is what makes the answer well defined: the Scharr gradient is not the exact
            derivative of the bilinear interpolant, so close to convergence the steps change the cost by
@@ -57,6 +58,9 @@ reduces/solves in float64):
            depended on the solver; with the slack every such step is taken, rejections are left for steps
            that really overshoot, and the loop contracts onto J^T r = 0 (scipy's root finder lands within
            3e-6 rad of it; 8.3 evaluations on average at 1080p against 11.8 without the step length).
+           The bound by c_0 keeps the slack from compounding on a poor start: a run that wanders (the slack accepts
+           up to 1 % more per step) could otherwise end above the cost it started from.  Returning the lowest-cost
+           accepted pose instead would not do: near convergence that pose is not the fixed point J^T r = 0.
            stop: |alpha d_w| < 5e-6 and |alpha d_t| < 1e-6 (accepted or rejected step), or 50 evaluations,
            or lambda > 1e6
   result   rvec = log(R), t, c, n, evaluations, status
@@ -200,6 +204,7 @@ def refine(pyramid: Sequence[np.ndarray], model: Model, kmat: np.ndarray, pose0:
     alpha = 1.0
     d_prev = None
     status = ST_MAX_EVALS
+    c_start = c
     if n == 0:
         status = ST_NONE
     while status == ST_MAX_EVALS and evals < max_evals:
@@ -228,7 +233,7 @@ def refine(pyramid: Sequence[np.ndarray], model: Model, kmat: np.ndarray, pose0:
         evals += 1
         nw, nt = math.sqrt(float(step[:3] @ step[:3])), math.sqrt(float(step[3:] @ step[3:]))
         small = nw < TOL_ROT and nt < TOL_TRANS
-        if n2 > 0 and c2 < c * (1.0 + ACCEPT_SLACK):
+        if n2 > 0 and c2 < c * (1.0 + ACCEPT_SLACK) and c2 <= c_start:
             rmat, t, hmat, b, c, n = r_try, t_try, h2, b2, c2, n2
             d_prev = d if lam <= LAMBDA0 else None
             lam = max(lam / 10.0, LAMBDA_MIN)
@@ -248,8 +253,12 @@ def refine(pyramid: Sequence[np.ndarray], model: Model, kmat: np.ndarray, pose0:
 def refine_multi(pyramid, model, kmat, poses0: np.ndarray, max_evals: int = MAX_EVALS):
     """Multi-hypothesis selection (SURVEY.md 8a row A7): lowest index within SELECT_TIE of the lowest 2c/n."""
     runs = [refine(pyramid, model, kmat, p, max_evals) for p in poses0]
+    return select(runs), runs
+
+
+def select(runs) -> int:
+    """Index of the winner among the results of refine() for the hypotheses of one frame (see refine_multi)."""
     score = np.array([2.0 * r["cost"] / r["n_valid"] if r["n_valid"] > 0 else np.inf for r in runs])
     if not np.isfinite(score).any():
-        return 0, runs
-    best = int(np.nonzero(score <= score.min() * (1.0 + SELECT_TIE))[0][0])
-    return best, runs
+        return 0
+    return int(np.nonzero(score <= score.min() * (1.0 + SELECT_TIE))[0][0])
