@@ -60,6 +60,7 @@ PROTOTYPES = {
     "agt_detect_tags": (_I, [_VP, _VP, _I, _I, _I64, _I64, _I, _I, _I, _I, _VP, _VP, _VP, _VP, _VP]),
     "agt_detect_tags_host": (_I, [_VP, _VP, _I, _I, _I, _I, _I, _VP, _VP, _VP, _VP, _VP]),
     "agt_detect_tags_roi": (_I, [_VP, _VP, _I, _I, _I64, _I64, _I, _VP, _I, _I, _I, _I, _VP, _VP, _VP, _VP, _VP]),
+    "agt_tag_quads": (_I, [_VP, _VP, _I, _I, _I64, _I64, _I, _VP, _I, _I, _I, _VP, _VP, _VP, _VP, _VP]),
     "agt_track_rects": (_I, [_VP, _VP, _D, _I, _I, _I, _VP, _I]),
     "agt_pack_detections": (_I, [_VP, _VP, _VP, _VP, _VP, _I, _VP, _I, C.c_float, _VP, _VP, _VP, _VP, _I]),
     "agt_draw_points": (_I, [_VP, _VP, _I, _I, _I64, _I64, _VP, _VP, _I, _I, _I, _I, _I, _I, _I, _I]),

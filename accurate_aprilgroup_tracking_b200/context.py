@@ -277,6 +277,31 @@ class AgtContext:
         out["n"].clamp_(max=max_tags)
         return out
 
+    def tag_quads(self, frames, width: Optional[int] = None, rects=None, max_quads: int = 64, refine_win: int = 4):
+        """The detector's first stage alone (threshold, components, quadrilateral fit) -> dict(n_comp [B] i32 components of area
+        >= 48 numbered, overflow [B] u8 (1: the global-memory union-find ran), n_quads [B] i32 (not clamped), quads
+        [B,max_quads,4,2] f32 clockwise in frame coordinates, win [B,max_quads] u8 the corner-refinement window of each quad);
+        slots beyond n_quads are undefined.  ``frames``: a Pyramid (level 0) or a uint8 tensor [B,H,pitch] on the device with
+        the frame ``width`` <= pitch (any pitch: the row reads take 16, 4 or 1 pixels at a time depending on the alignment)."""
+        t = self.torch
+        if isinstance(frames, Pyramid):
+            img, w, h, pitch, stride = frames.levels[0], frames.desc.width[0], frames.desc.height[0], frames.desc.pitch[0], frames.desc.frame_stride[0]
+        else:
+            if frames.dtype != t.uint8 or frames.dim() != 3 or not frames.is_cuda or frames.stride(2) != 1 or frames.stride(1) != frames.shape[2]:
+                raise ValueError("tag_quads: frames must be a device uint8 tensor [B,H,pitch] with contiguous rows")
+            img, h, pitch, stride = frames, int(frames.shape[1]), int(frames.shape[2]), int(frames.stride(0))
+            w = pitch if width is None else int(width)
+        b = int(img.shape[0])
+        out = {"n_comp": t.empty(b, dtype=t.int32, device=self.tdev), "overflow": t.empty(b, dtype=t.uint8, device=self.tdev),
+               "n_quads": t.empty(b, dtype=t.int32, device=self.tdev), "quads": t.empty((b, max_quads, 4, 2), dtype=t.float32, device=self.tdev),
+               "win": t.empty((b, max_quads), dtype=t.uint8, device=self.tdev)}
+        self._use_current_stream()
+        r = None if rects is None else self._dev(rects, t.int32)
+        self._check(self.lib.agt_tag_quads(self.h, self._p(img), int(w), int(h), int(pitch), int(stride), b, self._p(r) if r is not None else None,
+                                           int(r.shape[1]) if r is not None else 0, int(max_quads), int(refine_win), self._p(out["n_comp"]),
+                                           self._p(out["overflow"]), self._p(out["n_quads"]), self._p(out["quads"]), self._p(out["win"])))
+        return out
+
     def pack_detections(self, det, group_ids, min_margin: float = 50.0, out=None):
         """A0 on the device: the dict ``detect_tags`` returns -> (img_pts [B,4T,2] f32, valid [B,4T] u8, n_tags [B] i32, n_unknown
         [B] i32) indexed by the tags' positions in ``group_ids`` (the group's ids in JSON key order); detections with

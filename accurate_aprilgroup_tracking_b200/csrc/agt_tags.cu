@@ -211,7 +211,7 @@ extern "C" int agt_decode_tags(agt_ctx* ctx, const uint8_t* d_gray, int w, int h
 // =====================================================================================================================
 namespace {
 
-constexpr int MAX_COMPONENTS = 4096;      // per frame; what does not fit is ignored (counted)
+constexpr int MAX_COMPONENTS = 4096;      // per frame, components of area >= 48 (no smaller one can become a quad); what does not fit is ignored (counted)
 
 struct CompStats {
   int area;
@@ -524,8 +524,8 @@ __device__ __forceinline__ void ccl_union(int* L, int a, int b) {
 // component builds are walked at shared-memory latency: the same walk through global memory was three quarters of the
 // detector's component time) and roots get their component number.  What leaves the kernel is the component code of every run:
 // no pixel label is written or read on this path.  A frame with more entries or runs than the tables hold is flagged and goes
-// through ccl_merge_kernel, ccl_flatten_number_kernel and comp_stats_kernel instead (which return at once for every other
-// frame) and carries its codes in the pixel labels.
+// through ccl_merge_kernel, ccl_area_kernel and ccl_flatten_number_kernel instead (which return at once for every other frame)
+// and carries its codes in the pixel labels.
 constexpr int RUNS_THREADS = 1024, RUNS_ENT_PER = 4, RUNS_ENT_CAP = RUNS_ENT_PER * RUNS_THREADS, RUNS_RUN_CAP = 6 * RUNS_THREADS;
 
 // find with path halving: every node on the way is pointed at its grandparent.  Safe next to concurrent unions - a node that is
@@ -556,7 +556,7 @@ __global__ void __launch_bounds__(RUNS_THREADS, 1)
 ccl_runs_kernel(int w, int h, AGT_WIN_ARGS, const uint32_t* __restrict__ mask, int64_t mask_stride,
                 const int* __restrict__ n_entries, const int2* __restrict__ entries, const int* __restrict__ entry_of, int* __restrict__ n_comp,
                 CompStats* __restrict__ stats, uint8_t* __restrict__ overflow, int* __restrict__ run_code, int* __restrict__ ent_base,
-                int* __restrict__ label) {
+                int* __restrict__ label, int2* __restrict__ area_scratch) {
   __shared__ int s_parent[RUNS_RUN_CAP];
   __shared__ int s_base[RUNS_ENT_CAP];
   __shared__ int s_warp[RUNS_THREADS / 32];
@@ -570,9 +570,11 @@ ccl_runs_kernel(int w, int h, AGT_WIN_ARGS, const uint32_t* __restrict__ mask, i
   const int n = n_entries[f];
   // A frame that does not fit the tables goes through the pixel-level union-find (ccl_merge_kernel ...), which wants every dark
   // pixel labelled with the first pixel of its run inside the item - a run is then one tree of depth 1 and the merge pass joins
-  // runs, not pixels.  Only such frames pay for those labels.
+  // runs, not pixels.  Only such frames pay for those labels.  The area counter of each run's first pixel (ccl_area_kernel) starts
+  // at zero here.
   auto overflow_exit = [&]() {
     int* L = label + (int64_t)f * w * h;
+    int* A = reinterpret_cast<int*>(area_scratch + (int64_t)f * w * h);
     for (int e = tid; e < n; e += RUNS_THREADS) {
       const int2 v = E[e];
       const int y = v.x / chunks, i0 = y * win.ww + (v.x - y * chunks) * 32;
@@ -583,6 +585,7 @@ ccl_runs_kernel(int w, int h, AGT_WIN_ARGS, const uint32_t* __restrict__ mask, i
         mm &= mm - 1;
         const unsigned zeros_below = ~m & ((1u << bit) - 1u);
         L[i0 + bit] = i0 + (zeros_below ? 32 - __clz(zeros_below) : 0);
+        if (bit == 0 || !((m >> (bit - 1)) & 1u)) A[i0 + bit] = 0;
       }
     }
     if (tid == 0) overflow[f] = 1;
@@ -642,7 +645,7 @@ ccl_runs_kernel(int w, int h, AGT_WIN_ARGS, const uint32_t* __restrict__ mask, i
     }
   }
   __syncthreads();
-  // ---- roots, component numbers, codes
+  // ---- roots; every run points at its root, a root holds -1 - its area
   int root[RUNS_RUN_CAP / RUNS_THREADS];
 #pragma unroll
   for (int k = 0; k < RUNS_RUN_CAP / RUNS_THREADS; ++k) {
@@ -653,8 +656,30 @@ ccl_runs_kernel(int w, int h, AGT_WIN_ARGS, const uint32_t* __restrict__ mask, i
 #pragma unroll
   for (int k = 0; k < RUNS_RUN_CAP / RUNS_THREADS; ++k) {
     const int r = tid + k * RUNS_THREADS;
+    if (r < total) s_parent[r] = root[k] == r ? -1 : root[k];
+  }
+  __syncthreads();
+  for (int e = tid; e < n; e += RUNS_THREADS) {
+    unsigned mm = (unsigned)E[e].y;
+    int r = s_base[e];
+    while (mm) {
+      const int a = __ffs(mm) - 1;
+      const unsigned t = mm >> a;
+      const int len = t == 0xffffffffu ? 32 : __ffs(~t) - 1;
+      mm &= len == 32 ? 0u : ~(((1u << len) - 1u) << a);
+      const int p = s_parent[r];
+      atomicSub(&s_parent[p < 0 ? r : p], len);
+      ++r;
+    }
+  }
+  __syncthreads();
+  // ---- component numbers, codes: only a component that can become a quad (area >= 48, as far_pass and emit_quad ask) takes
+  // one of the MAX_COMPONENTS numbers, so that specks do not crowd out the tags
+#pragma unroll
+  for (int k = 0; k < RUNS_RUN_CAP / RUNS_THREADS; ++k) {
+    const int r = tid + k * RUNS_THREADS;
     if (r < total && root[k] == r) {
-      const int c = atomicAdd(&n_comp[f], 1);
+      const int c = -1 - s_parent[r] >= 48 ? atomicAdd(&n_comp[f], 1) : MAX_COMPONENTS;
       if (c < MAX_COMPONENTS) {
         CompStats& s = stats[(int64_t)f * MAX_COMPONENTS + c];
         s.area = 0; s.x0 = win.ww; s.y0 = win.hh; s.x1 = -1; s.y1 = -1; s.sx = 0; s.sy = 0; s.far0 = 0; s.far2 = 0; s.side_p = 0; s.side_n = 0;
@@ -704,14 +729,36 @@ __global__ void ccl_merge_kernel(int w, int h, AGT_WIN_ARGS, int* __restrict__ l
   }
 }
 
+// area of every component of an overflowing frame, at its root: each run adds its length (the counter of a root is the one
+// ccl_runs_kernel cleared at the run's first pixel; it lives in the boundary list's scratch, which nobody uses before
+// boundary_list_kernel)
+__global__ void ccl_area_kernel(int w, int h, AGT_WIN_ARGS, const int* __restrict__ label, const int* __restrict__ n_entries,
+                                const int2* __restrict__ entries, int64_t mask_stride, const uint8_t* __restrict__ overflow,
+                                int2* __restrict__ area_scratch) {
+  if (!overflow[blockIdx.y]) return;
+  const int* L = label + (int64_t)blockIdx.y * w * h;
+  int* A = reinterpret_cast<int*>(area_scratch + (int64_t)blockIdx.y * w * h);
+  const int2* E = entries + blockIdx.y * mask_stride;
+  AGT_WARP_SETUP
+  const int n = n_entries[f];
+  for (int e = warp0; e < n; e += nwarps) {
+    const Entry t = load_entry(E, e, n, chunks, win.ww, lane);
+    if (((t.m & ~(t.m << 1)) >> lane) & 1u) {
+      const unsigned rest = ~(t.m >> lane);
+      atomicAdd(&A[ccl_find(L, t.i)], rest == 0u ? 32 : __ffs(rest) - 1);
+    }
+  }
+}
+
 // every dark pixel is pointed at its root, and a root gets a component number on the spot: L[root] = -2 - number (numbers
-// beyond MAX_COMPONENTS are dropped: L[root] = -1 marks nothing).  A thread that walks through a root another thread has just
-// numbered sees a negative value there and stops: ccl_find.
+// beyond MAX_COMPONENTS are dropped: L[root] = -1 marks nothing; as in ccl_runs_kernel, only roots of area >= 48 are numbered).
+// A thread that walks through a root another thread has just numbered sees a negative value there and stops: ccl_find.
 __global__ void ccl_flatten_number_kernel(int w, int h, AGT_WIN_ARGS, int* __restrict__ label, const int* __restrict__ n_entries,
                                           const int2* __restrict__ entries, int64_t mask_stride, int* __restrict__ n_comp, CompStats* __restrict__ stats,
-                                          const uint8_t* __restrict__ overflow) {
+                                          const uint8_t* __restrict__ overflow, const int2* __restrict__ area_scratch) {
   if (!overflow[blockIdx.y]) return;
   int* L = label + (int64_t)blockIdx.y * w * h;
+  const int* A = reinterpret_cast<const int*>(area_scratch + (int64_t)blockIdx.y * w * h);
   const int2* E = entries + blockIdx.y * mask_stride;
   AGT_WARP_SETUP
   const int n = n_entries[f];
@@ -728,7 +775,7 @@ __global__ void ccl_flatten_number_kernel(int w, int h, AGT_WIN_ARGS, int* __res
       if (me[k] < 0) continue;
       const int i = t[k].i;
       if (me[k] == i) {
-        const int c = atomicAdd(&n_comp[f], 1);
+        const int c = A[i] >= 48 ? atomicAdd(&n_comp[f], 1) : MAX_COMPONENTS;
         if (c < MAX_COMPONENTS) {
           CompStats& s = stats[(int64_t)f * MAX_COMPONENTS + c];
           s.area = 0; s.x0 = win.ww; s.y0 = win.hh; s.x1 = -1; s.y1 = -1; s.sx = 0; s.sy = 0; s.far0 = 0; s.far2 = 0; s.side_p = 0; s.side_n = 0;
@@ -742,67 +789,21 @@ __global__ void ccl_flatten_number_kernel(int w, int h, AGT_WIN_ARGS, int* __res
   }
 }
 
-// before comp_stats_kernel: a root holds its code, every other dark pixel the index of its root
+// after ccl_flatten_number_kernel: a root holds its code, every other dark pixel the index of its root
 __device__ __forceinline__ int comp_of(const int* L, int l) {
   if (l == -1) return -1;
   if (l <= -2) return -2 - l;                   // a root
   const int r = L[l];
   return r <= -2 ? -2 - r : -1;
 }
-// after comp_stats_kernel every pixel of a numbered component holds the code itself
+// the code of a run in ccl_runs_kernel's table
 __device__ __forceinline__ int comp_code(int l) { return l <= -2 ? -2 - l : -1; }
-
-// all coordinates of the statistics are window coordinates.  The 32 pixels of a warp lie in one row and mostly in one component:
-// when every dark lane has the same component, the warp adds its totals with one set of atomics.  Every pixel is relabelled with
-// the code of its component, so that the later passes need one load per pixel (nobody else reads the label of a pixel that is
-// not a root).
-__global__ void comp_stats_kernel(int w, int h, AGT_WIN_ARGS, int* __restrict__ label, const int* __restrict__ n_entries,
-                                  const int2* __restrict__ entries, int64_t mask_stride, CompStats* __restrict__ stats,
-                                  const uint8_t* __restrict__ overflow) {
-  if (!overflow[blockIdx.y]) return;                   // ccl_runs_kernel has added up the runs already
-  int* L = label + (int64_t)blockIdx.y * w * h;
-  const int2* E = entries + blockIdx.y * mask_stride;
-  AGT_WARP_SETUP
-  const int n = n_entries[f];
-  for (int e = warp0 * 2; e < n; e += nwarps * 2) {
-    Entry t[2];
-    int me[2], cc[2];
-#pragma unroll
-    for (int k = 0; k < 2; ++k) {
-      t[k] = load_entry(E, e + k, n, chunks, win.ww, lane);
-      me[k] = t[k].dark ? L[t[k].i] : -1;
-    }
-#pragma unroll
-    for (int k = 0; k < 2; ++k) cc[k] = comp_of(L, me[k]);
-#pragma unroll
-    for (int k = 0; k < 2; ++k) {
-      const int c = cc[k], x = t[k].x, y = t[k].y;
-      const unsigned m = __ballot_sync(0xffffffffu, c >= 0);
-      if (m == 0) continue;
-      if (c >= 0 && me[k] >= 0) L[t[k].i] = -2 - c;
-      const int lead = __ffs(m) - 1, c0 = __shfl_sync(0xffffffffu, c, lead);
-      if (__all_sync(0xffffffffu, c < 0 || c == c0)) {
-        const int cnt = __popc(m), sumx = __reduce_add_sync(0xffffffffu, c >= 0 ? x : 0);
-        if (lane == lead) {
-          CompStats& s = stats[(int64_t)f * MAX_COMPONENTS + c0];
-          atomicAdd(&s.area, cnt);
-          atomicAdd(&s.sx, (unsigned long long)sumx); atomicAdd(&s.sy, (unsigned long long)y * cnt);
-          atomicMin(&s.x0, x); atomicMax(&s.x1, x - lane + 31 - __clz(m)); atomicMin(&s.y0, y); atomicMax(&s.y1, y);
-        }
-      } else if (c >= 0) {
-        CompStats& s = stats[(int64_t)f * MAX_COMPONENTS + c];
-        atomicAdd(&s.area, 1);
-        atomicAdd(&s.sx, (unsigned long long)x); atomicAdd(&s.sy, (unsigned long long)y);
-        atomicMin(&s.x0, x); atomicMin(&s.y0, y); atomicMax(&s.x1, x); atomicMax(&s.y1, y);
-      }
-    }
-  }
-}
 
 // The quadrilateral of a component comes from its boundary pixels (a dark pixel with a background pixel, or the edge of the
 // window, next to it) in three passes - 0: farthest from the centroid (c0); 1: farthest from c0 (c2); 2: farthest from the line
 // c0 c2 on each side.  boundary_list_kernel (a thread per entry, mask arithmetic only) lists the boundary pixels of a frame;
-// the three passes run a thread per listed pixel.
+// the three passes run a thread per listed pixel.  The same kernel adds up each component's statistics run by run, on either
+// union-find path (the run's code: from ccl_runs_kernel's table, or - frames that overflowed it - from the pixel labels).
 __global__ void boundary_list_kernel(int w, int h, AGT_WIN_ARGS, const int* __restrict__ label, const uint32_t* __restrict__ mask, int64_t mask_stride,
                                      const int* __restrict__ n_entries, const int2* __restrict__ entries, const uint8_t* __restrict__ overflow,
                                      const int* __restrict__ run_code, const int* __restrict__ ent_base, CompStats* __restrict__ stats,
@@ -848,12 +849,7 @@ __global__ void boundary_list_kernel(int w, int h, AGT_WIN_ARGS, const int* __re
       const int len = t == 0xffffffffu ? 32 : __ffs(~t) - 1;
       const unsigned bits = (len == 32 ? 0xffffffffu : (1u << len) - 1u) << a;
       mm &= ~bits;
-      if (by_label) {                                  // statistics came from comp_stats_kernel, codes sit in the labels
-        unsigned bb = bm & bits;
-        while (bb) { const int b = __ffs(bb) - 1; bb &= bb - 1; P[pos++] = make_int2(i0 + b, comp_code(L[i0 + b])); }
-        continue;
-      }
-      const int c = comp_code(code[base + r++]);
+      const int c = by_label ? comp_of(L, L[i0 + a]) : comp_code(code[base + r++]);
       if (c >= 0) {
         CompStats& st = stats[(int64_t)f * MAX_COMPONENTS + c];
         const int xa = xb + a;
@@ -954,7 +950,7 @@ __global__ void quad_emit_kernel(int w, int h, AGT_WIN_ARGS, const int* __restri
                                  float* __restrict__ quads, uint8_t* __restrict__ quad_valid, uint8_t* __restrict__ quad_win, int* __restrict__ n_quads,
                                  int max_quads, int refine_win, int32_t* __restrict__ out_n) {
   const int f = blockIdx.y, c = blockIdx.x * blockDim.x + threadIdx.x;
-  if (c == 0) out_n[f] = 0;
+  if (c == 0 && out_n != nullptr) out_n[f] = 0;
   if (c >= min(n_comp[f], MAX_COMPONENTS)) return;
   emit_quad(f, c, frame_window(rects, rect_stride, f, w, h), stats, quads, quad_valid, quad_win, n_quads, max_quads, refine_win);
 }
@@ -974,7 +970,7 @@ quad_fit_cluster_kernel(int w, int h, AGT_WIN_ARGS, const int* __restrict__ n_li
   const Win win = frame_window(rects, rect_stride, f, w, h);
   const int2* P = list + (int64_t)f * w * h;
   const int n = n_list[f];
-  if (t == 0) out_n[f] = 0;
+  if (t == 0 && out_n != nullptr) out_n[f] = 0;
   for (int pass = 0; pass < 3; ++pass) {
     far_pass(f, win.ww, P, n, stats, pass, t, FIT_CLUSTER * FIT_THREADS);
     __threadfence();
@@ -1035,52 +1031,55 @@ int agt_corner_subpix_windows(agt_ctx* ctx, const uint8_t* d_gray, int w, int h,
                               const uint8_t* d_valid, const uint8_t* d_win, float* d_out, int batch, int n_pts, int win, int max_iters,
                               double eps);
 
-extern "C" int agt_detect_tags_roi(agt_ctx* ctx, const uint8_t* d_gray, int w, int h, int64_t pitch, int64_t stride, int batch,
-                                   const int32_t* d_rects, int rect_stride, int max_tags, int max_hamming, int refine_win, int32_t* d_n_tags,
-                                   int32_t* d_ids, float* d_corners, float* d_margin, uint8_t* d_hamming) {
-  if (!ctx) return AGT_ERR_INVALID;
-  if (d_rects != nullptr && rect_stride < 4) AGT_FAIL(ctx, AGT_ERR_INVALID, "agt_detect_tags_roi: rect_stride < 4");
-  if (batch == 0) return AGT_OK;
-  if (!ctx->d_tag_codes) AGT_FAIL(ctx, AGT_ERR_NOT_READY, "agt_detect_tags: call agt_set_tag_family first");
-  if (!d_gray || !d_n_tags || !d_ids || !d_corners || batch < 0 || batch > 65535 || w < 16 || h < 16 || pitch < w || max_tags < 1 ||
-      max_tags > 1024 || (int64_t)w * h > 0x7fffffffLL || refine_win < 0 || refine_win > 7)
-    AGT_FAIL(ctx, AGT_ERR_INVALID, "agt_detect_tags: bad arguments");
-  const int max_quads = 4 * max_tags < 64 ? 64 : 4 * max_tags;
+// the detector's scratch: the pixel labels in slot 0, everything else in slot 1 (byte offsets into it)
+struct TagScratch {
+  int* label;
+  uint8_t* ws;
+  size_t o_stats, o_lohi, o_ncomp, o_nlist, o_nent, o_over, o_nquads, o_qvalid, o_win, o_quads, o_refined, o_id, o_rot, o_ham, o_margin, o_list,
+      o_mask, o_ent, o_pos, o_rcode, o_ebase, o_tiles, total;
+};
+
+// first half of the detector: threshold -> components -> farthest points -> quads (ws + o_quads, validity flags, refinement
+// windows; per frame the number of components numbered, the union-find that ran and the number of quads found).  out_n
+// (nullable): the detector's tag counters, cleared by the emission
+static int find_quads(agt_ctx* ctx, const uint8_t* d_gray, int w, int h, int64_t pitch, int64_t stride, int batch, const int32_t* d_rects,
+                      int rect_stride, int max_quads, int refine_win, int32_t* out_n, TagScratch& S) {
   const int64_t n = (int64_t)w * h, mask_stride = (int64_t)((w + 31) / 32) * h;
   const int64_t tile_stride = ((int64_t)((w + 31) / 32) * ((h + TILE - 1) / TILE) + 63) & ~(int64_t)63;
   // whole frames take the local white level, search windows one threshold each (agt_set_tag_threshold overrides)
   const bool local = ctx->tag_threshold == 2 || (ctx->tag_threshold == 0 && d_rects == nullptr);
-  int* label;
-  uint8_t* ws;
   int rc;
-  if ((rc = agt_scratch(ctx, 0, sizeof(int) * (size_t)n * batch, reinterpret_cast<void**>(&label)))) return rc;
-  const size_t o_stats = 0, o_lohi = o_stats + sizeof(CompStats) * (size_t)MAX_COMPONENTS * batch, o_ncomp = o_lohi + sizeof(int) * 2 * batch,
-               o_nlist = o_ncomp + sizeof(int) * batch, o_nent = o_nlist + sizeof(int) * batch, o_over = o_nent + sizeof(int) * batch, o_nquads = (o_over + (size_t)batch + 3) & ~(size_t)3,
-               o_qvalid = o_nquads + sizeof(int) * batch, o_win = o_qvalid + (size_t)max_quads * batch,             // everything up to here starts as zero
-               o_quads = (o_win + 4 * (size_t)max_quads * batch + 63) & ~(size_t)63, o_refined = o_quads + sizeof(float) * 8 * (size_t)max_quads * batch,
-               o_id = (o_refined + sizeof(float) * 8 * (size_t)max_quads * batch + 63) & ~(size_t)63,
-               o_rot = o_id + sizeof(int32_t) * (size_t)max_quads * batch, o_ham = o_rot + (size_t)max_quads * batch,
-               o_margin = (o_ham + (size_t)max_quads * batch + 63) & ~(size_t)63,
-               o_list = (o_margin + sizeof(float) * (size_t)max_quads * batch + 63) & ~(size_t)63, o_mask = o_list + sizeof(int2) * (size_t)n * batch,
-               o_ent = (o_mask + sizeof(uint32_t) * (size_t)mask_stride * batch + 63) & ~(size_t)63, o_pos = o_ent + sizeof(int2) * (size_t)mask_stride * batch,
-               o_rcode = o_pos + sizeof(int) * (size_t)mask_stride * batch, o_ebase = o_rcode + sizeof(int) * (size_t)RUNS_RUN_CAP * batch,
-               o_tiles = o_ebase + sizeof(int) * (size_t)RUNS_ENT_CAP * batch, total = o_tiles + (size_t)tile_stride * batch;
-  if ((rc = agt_scratch(ctx, 1, total, reinterpret_cast<void**>(&ws)))) return rc;
-  CompStats* stats = reinterpret_cast<CompStats*>(ws + o_stats);
-  int *lohi = reinterpret_cast<int*>(ws + o_lohi), *ncomp = reinterpret_cast<int*>(ws + o_ncomp), *nlist = reinterpret_cast<int*>(ws + o_nlist), *nent = reinterpret_cast<int*>(ws + o_nent),
-      *nquads = reinterpret_cast<int*>(ws + o_nquads);
-  float *quads = reinterpret_cast<float*>(ws + o_quads), *refined = reinterpret_cast<float*>(ws + o_refined);
-  uint8_t* qvalid = ws + o_qvalid;
-  int2* far_list = reinterpret_cast<int2*>(ws + o_list);
-  int2* entries = reinterpret_cast<int2*>(ws + o_ent);
-  uint32_t* mask = reinterpret_cast<uint32_t*>(ws + o_mask);
-  int* entry_of = reinterpret_cast<int*>(ws + o_pos);
-  uint8_t* overflow = ws + o_over;
-  int *run_code = reinterpret_cast<int*>(ws + o_rcode), *ent_base = reinterpret_cast<int*>(ws + o_ebase);
+  if ((rc = agt_scratch(ctx, 0, sizeof(int) * (size_t)n * batch, reinterpret_cast<void**>(&S.label)))) return rc;
+  S.o_stats = 0; S.o_lohi = S.o_stats + sizeof(CompStats) * (size_t)MAX_COMPONENTS * batch; S.o_ncomp = S.o_lohi + sizeof(int) * 2 * batch;
+  S.o_nlist = S.o_ncomp + sizeof(int) * batch; S.o_nent = S.o_nlist + sizeof(int) * batch; S.o_over = S.o_nent + sizeof(int) * batch;
+  S.o_nquads = (S.o_over + (size_t)batch + 3) & ~(size_t)3;
+  S.o_qvalid = S.o_nquads + sizeof(int) * batch; S.o_win = S.o_qvalid + (size_t)max_quads * batch;             // everything up to here starts as zero
+  S.o_quads = (S.o_win + 4 * (size_t)max_quads * batch + 63) & ~(size_t)63; S.o_refined = S.o_quads + sizeof(float) * 8 * (size_t)max_quads * batch;
+  S.o_id = (S.o_refined + sizeof(float) * 8 * (size_t)max_quads * batch + 63) & ~(size_t)63;
+  S.o_rot = S.o_id + sizeof(int32_t) * (size_t)max_quads * batch; S.o_ham = S.o_rot + (size_t)max_quads * batch;
+  S.o_margin = (S.o_ham + (size_t)max_quads * batch + 63) & ~(size_t)63;
+  S.o_list = (S.o_margin + sizeof(float) * (size_t)max_quads * batch + 63) & ~(size_t)63; S.o_mask = S.o_list + sizeof(int2) * (size_t)n * batch;
+  S.o_ent = (S.o_mask + sizeof(uint32_t) * (size_t)mask_stride * batch + 63) & ~(size_t)63; S.o_pos = S.o_ent + sizeof(int2) * (size_t)mask_stride * batch;
+  S.o_rcode = S.o_pos + sizeof(int) * (size_t)mask_stride * batch; S.o_ebase = S.o_rcode + sizeof(int) * (size_t)RUNS_RUN_CAP * batch;
+  S.o_tiles = S.o_ebase + sizeof(int) * (size_t)RUNS_ENT_CAP * batch; S.total = S.o_tiles + (size_t)tile_stride * batch;
+  if ((rc = agt_scratch(ctx, 1, S.total, reinterpret_cast<void**>(&S.ws)))) return rc;
+  uint8_t* ws = S.ws;
+  int* label = S.label;
+  CompStats* stats = reinterpret_cast<CompStats*>(ws + S.o_stats);
+  int *lohi = reinterpret_cast<int*>(ws + S.o_lohi), *ncomp = reinterpret_cast<int*>(ws + S.o_ncomp), *nlist = reinterpret_cast<int*>(ws + S.o_nlist),
+      *nent = reinterpret_cast<int*>(ws + S.o_nent), *nquads = reinterpret_cast<int*>(ws + S.o_nquads);
+  float* quads = reinterpret_cast<float*>(ws + S.o_quads);
+  uint8_t* qvalid = ws + S.o_qvalid;
+  int2* far_list = reinterpret_cast<int2*>(ws + S.o_list);
+  int2* entries = reinterpret_cast<int2*>(ws + S.o_ent);
+  uint32_t* mask = reinterpret_cast<uint32_t*>(ws + S.o_mask);
+  int* entry_of = reinterpret_cast<int*>(ws + S.o_pos);
+  uint8_t* overflow = ws + S.o_over;
+  int *run_code = reinterpret_cast<int*>(ws + S.o_rcode), *ent_base = reinterpret_cast<int*>(ws + S.o_ebase);
   cudaStream_t st = ctx->stream;
   // one memset: darkest / brightest pixel (stored so that both start as 0), counters, overflow flags, validity flags and
   // refinement windows of the quads; the tag counters are cleared by the quad emission
-  AGT_CUDA(ctx, cudaMemsetAsync(ws + o_lohi, 0, o_quads - o_lohi, st));
+  AGT_CUDA(ctx, cudaMemsetAsync(ws + S.o_lohi, 0, S.o_quads - S.o_lohi, st));
   // grid-stride over the pixels of each frame's window; with windows (usually a few percent of the frame) a smaller grid per frame
   // (whole frames: 32 CTAs per SM over the batch - a grid sized for one frame, times 64 frames, spent its time launching CTAs
   // that had nothing to do: 174 + 188 us for min/max + threshold of 64 1080p frames)
@@ -1091,16 +1090,16 @@ extern "C" int agt_detect_tags_roi(agt_ctx* ctx, const uint8_t* d_gray, int w, i
   // (both passes of a frame by one CTA of 1024 threads - one launch, tile maxima in shared memory, the second read from the L2 -
   // measured slower: 48 against 13 + 21 us per 64 windows, 293 against 57 + 80 us per 64 whole frames; the threshold pass is
   // instruction work - dark bits, runs, first labels - that one SM per frame does not get through)
-  uint8_t* tiles = local ? ws + o_tiles : nullptr;
+  uint8_t* tiles = local ? ws + S.o_tiles : nullptr;
   if (local) tile_max_kernel<<<grid, 256, 0, st>>>(d_gray, w, h, pitch, stride, d_rects, rect_stride, lohi, tiles, tile_stride);
   else frame_minmax_kernel<<<grid, 256, 0, st>>>(d_gray, w, h, pitch, stride, d_rects, rect_stride, lohi);
   ccl_init_kernel<<<grid, 256, 0, st>>>(d_gray, w, h, pitch, stride, d_rects, rect_stride, lohi, tiles, tile_stride, mask, mask_stride, nent, entries,
                                        entry_of);
   ccl_runs_kernel<<<(unsigned)batch, RUNS_THREADS, 0, st>>>(w, h, d_rects, rect_stride, mask, mask_stride, nent, entries, entry_of, ncomp, stats,
-                                                           overflow, run_code, ent_base, label);
+                                                           overflow, run_code, ent_base, label, far_list);
   ccl_merge_kernel<<<grid_ne, 256, 0, st>>>(w, h, d_rects, rect_stride, label, mask, mask_stride, nent, entries, overflow);
-  ccl_flatten_number_kernel<<<grid_ne, 256, 0, st>>>(w, h, d_rects, rect_stride, label, nent, entries, mask_stride, ncomp, stats, overflow);
-  comp_stats_kernel<<<grid_ne, 256, 0, st>>>(w, h, d_rects, rect_stride, label, nent, entries, mask_stride, stats, overflow);
+  ccl_area_kernel<<<grid_ne, 256, 0, st>>>(w, h, d_rects, rect_stride, label, nent, entries, mask_stride, overflow, far_list);
+  ccl_flatten_number_kernel<<<grid_ne, 256, 0, st>>>(w, h, d_rects, rect_stride, label, nent, entries, mask_stride, ncomp, stats, overflow, far_list);
   boundary_list_kernel<<<grid_ne, 256, 0, st>>>(w, h, d_rects, rect_stride, label, mask, mask_stride, nent, entries, overflow, run_code, ent_base, stats,
                                                 nlist, far_list);
   if (batch >= 8) {
@@ -1113,27 +1112,72 @@ extern "C" int agt_detect_tags_roi(agt_ctx* ctx, const uint8_t* d_gray, int w, i
     at[0].val.clusterDim.x = FIT_CLUSTER; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
     cfg.attrs = at; cfg.numAttrs = 1;
     const int* c_nlist = nlist; const int2* c_list = far_list; const int* c_ncomp = ncomp;
-    uint8_t* qwin = ws + o_win;
+    uint8_t* qwin = ws + S.o_win;
     const cudaError_t e = cudaLaunchKernelEx(&cfg, quad_fit_cluster_kernel, w, h, d_rects, rect_stride, c_nlist, c_list, c_ncomp, stats, quads,
-                                             qvalid, qwin, nquads, max_quads, refine_win, d_n_tags);
+                                             qvalid, qwin, nquads, max_quads, refine_win, out_n);
     if (e != cudaSuccess) AGT_FAIL(ctx, AGT_ERR_CUDA, "agt_detect_tags: cluster launch failed: %s", cudaGetErrorString(e));
   } else {
     for (int pass = 0; pass < 3; ++pass) comp_far_kernel<<<grid_ne, 256, 0, st>>>(w, h, d_rects, rect_stride, nlist, far_list, stats, pass);
     quad_emit_kernel<<<dim3(MAX_COMPONENTS / 128, (unsigned)batch), 128, 0, st>>>(w, h, d_rects, rect_stride, ncomp, stats, quads, qvalid,
-                                                                                     ws + o_win, nquads, max_quads, refine_win, d_n_tags);
+                                                                                     ws + S.o_win, nquads, max_quads, refine_win, out_n);
   }
   AGT_LAUNCH_CHECK(ctx);
-  const float* use = quads;
+  return AGT_OK;
+}
+
+static bool tag_args_ok(const uint8_t* d_gray, int w, int h, int64_t pitch, int batch, int refine_win) {
+  return d_gray && batch > 0 && batch <= 65535 && w >= 16 && h >= 16 && pitch >= w && (int64_t)w * h <= 0x7fffffffLL && refine_win >= 0 &&
+         refine_win <= 7;
+}
+
+extern "C" int agt_tag_quads(agt_ctx* ctx, const uint8_t* d_gray, int w, int h, int64_t pitch, int64_t stride, int batch, const int32_t* d_rects,
+                             int rect_stride, int max_quads, int refine_win, int32_t* d_n_comp, uint8_t* d_overflow, int32_t* d_n_quads,
+                             float* d_quads, uint8_t* d_quad_win) {
+  if (!ctx) return AGT_ERR_INVALID;
+  if (d_rects != nullptr && rect_stride < 4) AGT_FAIL(ctx, AGT_ERR_INVALID, "agt_tag_quads: rect_stride < 4");
+  if (batch == 0) return AGT_OK;
+  if (!tag_args_ok(d_gray, w, h, pitch, batch, refine_win) || max_quads < 1 || max_quads > MAX_COMPONENTS || !d_n_comp || !d_overflow || !d_n_quads ||
+      !d_quads || !d_quad_win)
+    AGT_FAIL(ctx, AGT_ERR_INVALID, "agt_tag_quads: bad arguments");
+  TagScratch S;
+  int rc;
+  if ((rc = find_quads(ctx, d_gray, w, h, pitch, stride, batch, d_rects, rect_stride, max_quads, refine_win, nullptr, S))) return rc;
+  cudaStream_t st = ctx->stream;
+  AGT_CUDA(ctx, cudaMemcpyAsync(d_n_comp, S.ws + S.o_ncomp, sizeof(int32_t) * (size_t)batch, cudaMemcpyDeviceToDevice, st));
+  AGT_CUDA(ctx, cudaMemcpyAsync(d_overflow, S.ws + S.o_over, (size_t)batch, cudaMemcpyDeviceToDevice, st));
+  AGT_CUDA(ctx, cudaMemcpyAsync(d_n_quads, S.ws + S.o_nquads, sizeof(int32_t) * (size_t)batch, cudaMemcpyDeviceToDevice, st));
+  AGT_CUDA(ctx, cudaMemcpyAsync(d_quads, S.ws + S.o_quads, sizeof(float) * 8 * (size_t)max_quads * batch, cudaMemcpyDeviceToDevice, st));
+  // (the detector keeps the window once per corner)
+  AGT_CUDA(ctx, cudaMemcpy2DAsync(d_quad_win, 1, S.ws + S.o_win, 4, 1, (size_t)max_quads * batch, cudaMemcpyDeviceToDevice, st));
+  return AGT_OK;
+}
+
+extern "C" int agt_detect_tags_roi(agt_ctx* ctx, const uint8_t* d_gray, int w, int h, int64_t pitch, int64_t stride, int batch,
+                                   const int32_t* d_rects, int rect_stride, int max_tags, int max_hamming, int refine_win, int32_t* d_n_tags,
+                                   int32_t* d_ids, float* d_corners, float* d_margin, uint8_t* d_hamming) {
+  if (!ctx) return AGT_ERR_INVALID;
+  if (d_rects != nullptr && rect_stride < 4) AGT_FAIL(ctx, AGT_ERR_INVALID, "agt_detect_tags_roi: rect_stride < 4");
+  if (batch == 0) return AGT_OK;
+  if (!ctx->d_tag_codes) AGT_FAIL(ctx, AGT_ERR_NOT_READY, "agt_detect_tags: call agt_set_tag_family first");
+  if (!tag_args_ok(d_gray, w, h, pitch, batch, refine_win) || !d_n_tags || !d_ids || !d_corners || max_tags < 1 || max_tags > 1024)
+    AGT_FAIL(ctx, AGT_ERR_INVALID, "agt_detect_tags: bad arguments");
+  const int max_quads = 4 * max_tags < 64 ? 64 : 4 * max_tags;
+  TagScratch S;
+  int rc;
+  if ((rc = find_quads(ctx, d_gray, w, h, pitch, stride, batch, d_rects, rect_stride, max_quads, refine_win, d_n_tags, S))) return rc;
+  uint8_t* ws = S.ws;
+  const float* use = reinterpret_cast<const float*>(ws + S.o_quads);
   if (refine_win > 0) {
     // only the corners of emitted quads (the validity flag of a quad, four times), each with its own window
-    if ((rc = agt_corner_subpix_windows(ctx, d_gray, w, h, pitch, stride, quads, ws + o_win, ws + o_win, refined, batch, 4 * max_quads,
+    float* refined = reinterpret_cast<float*>(ws + S.o_refined);
+    if ((rc = agt_corner_subpix_windows(ctx, d_gray, w, h, pitch, stride, use, ws + S.o_win, ws + S.o_win, refined, batch, 4 * max_quads,
                                         refine_win, TAG_SUBPIX_ITERS, 1e-3)))
       return rc;
     use = refined;
   }
   // identification; the quads that decode go straight to the caller's list (no collection pass)
-  if ((rc = decode_tags(ctx, d_gray, w, h, pitch, stride, use, qvalid, reinterpret_cast<int32_t*>(ws + o_id), ws + o_rot, ws + o_ham,
-                        reinterpret_cast<float*>(ws + o_margin), batch, max_quads, max_hamming,
+  if ((rc = decode_tags(ctx, d_gray, w, h, pitch, stride, use, ws + S.o_qvalid, reinterpret_cast<int32_t*>(ws + S.o_id), ws + S.o_rot, ws + S.o_ham,
+                        reinterpret_cast<float*>(ws + S.o_margin), batch, max_quads, max_hamming,
                         TagSink{d_n_tags, d_ids, d_corners, d_margin, d_hamming, max_tags})))
     return rc;
   AGT_LAUNCH_CHECK(ctx);

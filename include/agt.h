@@ -155,6 +155,15 @@ int agt_set_tag_threshold(agt_ctx* ctx, int mode);
 int agt_detect_tags_roi(agt_ctx* ctx, const uint8_t* d_gray, int w, int h, int64_t pitch, int64_t stride, int batch,
                         const int32_t* d_rects, int rect_stride, int max_tags, int max_hamming, int refine_win, int32_t* d_n_tags,
                         int32_t* d_ids, float* d_corners, float* d_margin, uint8_t* d_hamming);
+/* The first stage of agt_detect_tags_roi on its own, up to and including the quad emission (same arguments; the detector's
+ * max_quads is max(64, 4 max_tags), here 1..4096): per frame d_n_comp = dark components of area >= 48 that were numbered (not
+ * clamped: beyond 4096 some are dropped), d_overflow = 1 if the frame took the global-memory union-find, d_n_quads = quads found
+ * (not clamped to max_quads), d_quads [batch][max_quads][4][2] (clockwise on the screen, frame coordinates; slot order not
+ * defined, slots beyond d_n_quads undefined) and d_quad_win [batch][max_quads], the window agt_detect_tags refines each quad's
+ * corners with.  Semantics: oracle/tag_oracle.py:quads_np. */
+int agt_tag_quads(agt_ctx* ctx, const uint8_t* d_gray, int w, int h, int64_t pitch, int64_t stride, int batch, const int32_t* d_rects,
+                  int rect_stride, int max_quads, int refine_win, int32_t* d_n_comp, uint8_t* d_overflow, int32_t* d_n_quads,
+                  float* d_quads, uint8_t* d_quad_win);
 /* Search windows from the stream states (see agt_ape_prepare): the image of a sphere of `radius` metres around the group's origin
  * at the predicted pose (the extrinsic guess, detect_pose.py:553-566), else at the last accepted pose, grown by `margin` pixels;
  * streams without a pose get the empty rectangle (= whole frame).  d_rects [batch][4] int32, 16-byte aligned. */

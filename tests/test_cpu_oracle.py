@@ -296,3 +296,66 @@ def test_pack_detections_host_rules():
     assert valid[2].tolist() == [0] * 8 + [1] * 4 + [0] * 4
     with pytest.raises(KeyError):
         pack_detections([[(5, c)]], group)
+
+
+# the detector's first stage (tag_oracle.quads_np) and the case set of tests/test_gpu_tag_quads.py
+@pytest.fixture(scope="module")
+def tag_quad_cases():
+    from tests import tag_quad_cases
+    return tag_quad_cases.build()
+
+
+def test_tag_quad_case_set_hits_its_targets(tag_quad_cases):
+    missed = [c["name"] for c in tag_quad_cases if not c["target"](c["oracle"])]
+    assert not missed, missed
+
+
+def test_quads_np_components_equal_opencv(tag_quad_cases):
+    """The components of quads_np (scipy.ndimage.label) against cv2.connectedComponentsWithStats with 4-connectivity: count,
+    areas, bounding boxes and centroids identical on the whole case set."""
+    import cv2
+    for c in tag_quad_cases:
+        r = c["oracle"]
+        n, lab, st, cen = cv2.connectedComponentsWithStats(r["dark"].astype(np.uint8), connectivity=4)
+        assert n - 1 == r["n_all"], c["name"]
+        bb = r["bbox"][1:]
+        ours = np.column_stack([bb[:, 0], bb[:, 1], bb[:, 2] - bb[:, 0] + 1, bb[:, 3] - bb[:, 1] + 1, r["area"][1:]])
+        order_cv = np.lexsort(st[1:].T[::-1])
+        order_np = np.lexsort(ours.T[::-1])
+        assert np.array_equal(st[1:][order_cv], ours[order_np]), c["name"]
+        cen_np = np.column_stack([r["sx"][1:] / r["area"][1:], r["sy"][1:] / r["area"][1:]])
+        assert np.array_equal(cen[1:][order_cv], cen_np[order_np]), c["name"]
+
+
+def test_quads_np_far_points_equal_brute_force(tag_quad_cases):
+    """The three farthest-point passes of quads_np (vectorised, segment maxima of packed keys) against a loop over every pixel of
+    each component (boundary test per pixel, keys compared as (value, pixel index) pairs: the larger index wins a tie)."""
+    F = np.float32
+    checked = 0
+    for c in tag_quad_cases:
+        r = c["oracle"]
+        lab, dark = r["labels"], r["dark"]
+        hh, ww = dark.shape
+        comps = [k for k in r["far"]][:40]
+        for k in comps:
+            ys, xs = np.nonzero(lab == k)
+            px = []
+            for y, x in zip(ys.tolist(), xs.tolist()):
+                nb = [(y - 1, x), (y + 1, x), (y, x - 1), (y, x + 1)]
+                if any(not (0 <= v < hh and 0 <= u < ww) or not dark[v, u] for v, u in nb):
+                    px.append((y, x, y * ww + x))
+            cx, cy = F(int(r["sx"][k]) / int(r["area"][k])), F(int(r["sy"][k]) / int(r["area"][k]))
+            best = max(((F(F(F(x) - cx) * F(F(x) - cx)) + F(F(F(y) - cy) * F(F(y) - cy)), i) for y, x, i in px))
+            alts = r["far"][k]
+            assert best[1] in {a[0] for a in alts}, (c["name"], k)
+            p0, sp, p2, sn, _ = alts[0]
+            x0, y0 = p0 % ww, p0 // ww
+            far2 = max(((x - x0) ** 2 + (y - y0) ** 2, i) for y, x, i in px)
+            assert far2[1] == p2, (c["name"], k)
+            x2, y2 = p2 % ww, p2 // ww
+            d = [((x2 - x0) * (y - y0) - (y2 - y0) * (x - x0), i) for y, x, i in px]
+            pos = max(((v, i) for v, i in d if v > 0), default=(0, 0))
+            neg = max(((-v, i) for v, i in d if v < 0), default=(0, 0))
+            assert (pos[1], neg[1]) == (sp, sn), (c["name"], k)
+            checked += 1
+    assert checked >= 200
