@@ -145,7 +145,7 @@ __device__ __forceinline__ void rodrigues_step(const double w[3], double R[9]) {
 }
 
 // shared-window address kept opaque so that it stays in one register instead of being re-derived in the loop;
-// the loads below carry a memory clobber so that the compiler keeps (and orders) the C++ stores they read
+// the pose load carries a memory clobber so that the compiler keeps (and orders) the C++ stores it reads
 __device__ __forceinline__ uint32_t smem_addr(const void* p) {
   uint32_t a = (uint32_t)__cvta_generic_to_shared(p), o;
   asm volatile("mov.u32 %0, %1;" : "=r"(o) : "r"(a));
@@ -156,9 +156,11 @@ __device__ __forceinline__ double2 lds_f64x2(uint32_t a) {
   asm volatile("ld.shared.v2.f64 {%0, %1}, [%2];" : "=d"(v.x), "=d"(v.y) : "r"(a) : "memory");
   return v;
 }
+// A tile word: a plain load the compiler may schedule freely.  The tile is written once, before the barrier that ends
+// staging, and the address of every read depends on the pose the sample loop loads after that barrier.
 __device__ __forceinline__ uint32_t lds_u32(uint32_t a) {
   uint32_t v;
-  asm volatile("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(a) : "memory");
+  asm("ld.shared.u32 %0, [%1];" : "=r"(v) : "r"(a));
   return v;
 }
 
@@ -193,6 +195,18 @@ constexpr int C_SM1 = (int)0x030A0300;      // (  0,  3, 10,  3)   horizontal sm
 constexpr int C_SM0_NEG = (int)0x00FDF6FD;  // ( -3,-10, -3,  0)
 constexpr int C_SM1_NEG = (int)0xFDF6FD00;  // (  0, -3,-10, -3)
 __constant__ int kCoef[8] = {C_DX0_3, C_DX0_10, C_DX1_3, C_DX1_10, C_SM0, C_SM1, C_SM0_NEG, C_SM1_NEG};
+
+// One sample projected at the trial pose: what the footprint test, the fetch and the normal-equation products need
+struct DprSample {
+  f32x2 Yxy;       // float32 lever arm R x (x, y)
+  f32x2 XY;        // camera-frame (X, Y)
+  f32x2 ab;        // bilinear fractions of (ul, vl)
+  float Yz, Z32;   // lever arm z, camera-frame depth
+  float iz;        // approximate 1 / Z32
+  float w;         // model intensity of the sample
+  int lx, ly;      // footprint origin relative to the staged tile
+  bool depth_ok;
+};
 
 // Per-refinement setup that depends only on the initial pose, computed by one thread per refinement in a launch of its
 // own (dpr_prep_kernel) instead of by thread 0 of every CTA while 255 threads wait: pyramid level and ROI plan
@@ -529,7 +543,6 @@ dpr_kernel(agt_pyramid pyr, agt_camera cam, const float4* __restrict__ samples, 
     }
   }
 
-  const int n_act_samples = S.act_prefix[S.n_active];
   const float fx = S.fx, fy = S.fy, gsc = S.gscale;
   const int lw = S.lw, lh = S.lh, tx0 = S.tx0, ty0 = S.ty0;
   const int64_t lpitch = S.lpitch;
@@ -556,27 +569,31 @@ dpr_kernel(agt_pyramid pyr, agt_camera cam, const float4* __restrict__ samples, 
     const f32x2* Rp = reinterpret_cast<const f32x2*>(S.Rf);
     const f32x2 R03 = Rp[0], R14 = Rp[1], R25 = Rp[2], t01 = Rp[3];
     const float R6 = S.Rf[8], R7 = S.Rf[9], R8 = S.Rf[10], t2 = S.Rf[11];
-    // One sample: projection, footprint fetch, Scharr taps, residual, Jacobian, normal-equation products.
-    auto eval_sample = [&](const float4 sm) {
+    // A sample is projected (project), its 4x4 footprint fetched from the staged tile (fetch_tile) or, when the footprint
+    // leaves the tile, by eval_sample's global-memory path, and its products added to the sums (accumulate).  Every
+    // float32 operation of these is written out (fma2 / fmaf / __fmul_rn): the fast pair body below and eval_sample then
+    // round alike whatever the compiler would contract, and the sums come out the same whichever path a sample takes.
+    auto project = [&](const float4 sm) {
+      DprSample q;
       // float32 lever arm Y = R x for the Jacobian and the reciprocal-depth seed (rounding of these only perturbs
       // the LM step, not the cost)
-      const f32x2 Yxy = fma2(R25, bc2(sm.z), fma2(R14, bc2(sm.y), mul2(R03, bc2(sm.x))));
-      const float Yz = fmaf(R8, sm.z, fmaf(R7, sm.y, R6 * sm.x));
-      const float Z32 = Yz + t2;
-      float iz;
-      asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(iz) : "f"(Z32));             // MUFU.RCP: Jacobian + Newton seed
+      q.Yxy = fma2(R25, bc2(sm.z), fma2(R14, bc2(sm.y), mul2(R03, bc2(sm.x))));
+      q.Yz = fmaf(R8, sm.z, fmaf(R7, sm.y, __fmul_rn(R6, sm.x)));
+      q.Z32 = __fadd_rn(q.Yz, t2);
+      asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(q.iz) : "f"(q.Z32));         // MUFU.RCP: Jacobian + Newton seed
+      q.XY = add2(q.Yxy, t01);
 #if AGT_DPR_F32_PROJECTION
       // Projection in float32.  Round 1 needed float64 here: its LM accepted a step only if the cost went down, near convergence
       // that compares costs 1e-6 apart, and float32 pixel coordinates (ulp 1e-4 px at 1080p) flipped 20 % of those decisions.
       // The loop now accepts within a 1e-2 slack and contracts onto J^T r = 0 (oracle/dpr_oracle.py), so that noise only moves
       // the fixed point by ~1e-8 rad, and the projection is the camera-frame (X, Y) the Jacobian needs anyway times a Newton-
       // refined reciprocal depth: 11 instructions instead of 28 (13 of them DFMA at two issue cycles each).
-      const float iz1 = iz * fmaf(-Z32, iz, 2.f);
-      const f32x2 XY = add2(Yxy, t01);
-      const f32x2 uv = fma2(mul2(XY, fl2), bc2(iz1), cl2);                 // (ul, vl)
+      const float iz1 = __fmul_rn(q.iz, fmaf(-q.Z32, q.iz, 2.f));
+      const f32x2 uv = fma2(mul2(q.XY, fl2), bc2(iz1), cl2);              // (ul, vl)
       const float fu = floorf(lo2(uv)), fv = floorf(hi2(uv));
-      const int lx = __float2int_rd(lo2(uv)) - xoff, ly = __float2int_rd(hi2(uv)) - yoff;   // footprint origin in the tile
-      const bool depth_ok = Z32 > 1e-6f;
+      q.lx = __float2int_rd(lo2(uv)) - xoff; q.ly = __float2int_rd(hi2(uv)) - yoff;   // footprint origin in the tile
+      q.depth_ok = q.Z32 > 1e-6f;
+      q.ab = add2(uv, pk2(-fu, -fv));                                      // (a, b) = fractions of (ul, vl)
 #else
       // Projection in float64: the accept/reject decisions of the LM loop compare costs that differ by ~1e-6
       // relative near convergence; float32 pixel coordinates (ulp 6e-5 px at 1080p) add ~1e-6 of noise to the
@@ -589,43 +606,36 @@ dpr_kernel(agt_pyramid pyr, agt_camera cam, const float4* __restrict__ samples, 
       const double dX = fma(p01.x, sx, fma(p01.y, sy, fma(p23.x, sz, p8t.y)));
       const double dY = fma(p23.y, sx, fma(p45.x, sy, fma(p45.y, sz, ptt.x)));
       const double dZ = fma(p67.x, sx, fma(p67.y, sy, fma(p8t.x, sz, ptt.y)));
-      double r0 = (double)iz;                         // 2^-22 relative; one Newton step -> 2^-44 (4e-11 px at 1080p)
+      double r0 = (double)q.iz;                       // 2^-22 relative; one Newton step -> 2^-44 (4e-11 px at 1080p)
       r0 = r0 * (2.0 - dZ * r0);
       // floor + fraction without conversions or float64 compares: ul + 1.5 * 2^20 (one FMA rounding down) leaves
       // floor(ul) in the low bits of the high mantissa word and the fraction, scaled by 2^32, in the low word;
       // NaN / Inf / |ul| >= 2^19 give a high word far outside any image
       const double kMagic = 1572864.0;
       const double tu = __fma_rd(dX, r0, kMagic), tv = __fma_rd(dY, r0, kMagic);
-      const int lx = __double2hiint(tu) - xbias, ly = __double2hiint(tv) - ybias;     // footprint origin in the tile
-      const bool depth_ok = dZ > 1e-6;
+      q.lx = __double2hiint(tu) - xbias; q.ly = __double2hiint(tv) - ybias;     // footprint origin in the tile
+      q.depth_ok = dZ > 1e-6;
+      q.ab = mul2(pk2((float)(uint32_t)__double2loint(tu), (float)(uint32_t)__double2loint(tv)), bc2(2.3283064365386963e-10f));
 #endif
-      // 4x4 footprint rows y0-1..y0+2, columns x0-1..x0+2
-      uint32_t row[4];
-      if (Z32 > 2e-6f && (uint32_t)lx < tw_m3 && (uint32_t)ly < th_m3) {
-        // (float32 depth above 2e-6 implies float64 depth above 1e-6; the tile lies inside the level image, so a
-        // footprint inside the tile is a valid sample)
-        const uint32_t a0 = sT + ly * TILE_PITCH + (lx & ~3);
-        const uint32_t sel = 0x3210 + 0x1111 * (lx & 3);
+      q.w = sm.w;
+      return q;
+    };
+    // (float32 depth above 2e-6 implies float64 depth above 1e-6; the tile lies inside the level image, so a footprint
+    // inside the tile is a valid sample)
+    auto in_tile = [&](const DprSample& q) { return q.Z32 > 2e-6f && (uint32_t)q.lx < tw_m3 && (uint32_t)q.ly < th_m3; };
+    // 4x4 footprint rows y0-1..y0+2, columns x0-1..x0+2: two aligned words and a byte permute per row
+    auto fetch_tile = [&](const DprSample& q, uint32_t row[4]) {
+      const uint32_t a0 = sT + q.ly * TILE_PITCH + (q.lx & ~3);
+      const uint32_t sel = 0x3210 + 0x1111 * (q.lx & 3);
 #pragma unroll
-        for (int r = 0; r < 4; ++r) row[r] = __byte_perm(lds_u32(a0 + r * TILE_PITCH), lds_u32(a0 + r * TILE_PITCH + 4), sel);
-      } else {
-        const int x0 = lx + tx0 + 1, y0 = ly + ty0 + 1;
-        // valid <=> z > 1e-6 and 1 <= floor(ul) <= lw-3 and 1 <= floor(vl) <= lh-3
-        if (!depth_ok || x0 < 1 || x0 > lw - 3 || y0 < 1 || y0 > lh - 3) return;
-        if (x0 - 1 < S.rx0 || y0 - 1 < S.ry0 || x0 + 3 > S.rx1 || y0 + 3 > S.ry1) S.left_roi = 1;   // benign race: all write 1
-        const uint8_t* g = limg + (int64_t)(y0 - 1) * lpitch + (x0 - 1);
-#pragma unroll
-        for (int r = 0; r < 4; ++r) row[r] = ld4_global(g + r * lpitch);
-      }
-      // bilinear weights; (a, b) = fractions of (ul, vl)
-#if AGT_DPR_F32_PROJECTION
-      const f32x2 ab = add2(uv, pk2(-fu, -fv));
-#else
-      const f32x2 ab = mul2(pk2((float)(uint32_t)__double2loint(tu), (float)(uint32_t)__double2loint(tv)), bc2(2.3283064365386963e-10f));
-#endif
+      for (int r = 0; r < 4; ++r) row[r] = __byte_perm(lds_u32(a0 + r * TILE_PITCH), lds_u32(a0 + r * TILE_PITCH + 4), sel);
+    };
+    // Scharr taps, bilinear intensity and gradient, residual, Jacobian, normal-equation products
+    auto accumulate = [&](const DprSample& q, const uint32_t row[4]) {
+      const f32x2 ab = q.ab;
       const f32x2 omab = fma2(ab, bc2(-1.f), bc2(1.f));                     // (1-a, 1-b)
       const f32x2 wx = mul2(ab, swap2(omab));                               // (w01, w10) = (a (1-b), b (1-a))
-      const float w00 = lo2(omab) * hi2(omab), w11 = lo2(ab) * hi2(ab), w01 = lo2(wx), w10 = hi2(wx);
+      const float w00 = __fmul_rn(lo2(omab), hi2(omab)), w11 = __fmul_rn(lo2(ab), hi2(ab)), w01 = lo2(wx), w10 = hi2(wx);
       // Scharr at (x0,y0) (x0+1,y0) (x0,y0+1) (x0+1,y0+1): the [3 10 3] row weights are folded into the byte
       // coefficients and the three rows are chained through the dp4a accumulator, which starts at the bit pattern of
       // 1.5 * 2^23: the integer sum lands in the mantissa and one packed subtraction turns two taps into floats
@@ -641,18 +651,15 @@ dpr_kernel(agt_pyramid pyr, agt_camera cam, const float4* __restrict__ samples, 
                                  dp4c(row[3], cSM1, dp4c(row[1], cSM1_NEG, kB))), kNegBias);
       const float i00 = (float)((row[1] >> 8) & 0xffu), i01 = (float)((row[1] >> 16) & 0xffu);
       const float i10 = (float)((row[2] >> 8) & 0xffu), i11 = (float)((row[2] >> 16) & 0xffu);
-      const float I = w00 * i00 + w01 * i01 + w10 * i10 + w11 * i11;
+      const float I = fmaf(w11, i11, fmaf(w10, i10, fmaf(w00, i00, __fmul_rn(w01, i01))));
       const f32x2 G = fma2(bc2(w11), g11, fma2(bc2(w10), g10, fma2(bc2(w01), g01, mul2(bc2(w00), g00))));   // (Gx, Gy) * 32 * 2^l
-      const float r = I - sm.w;
-      const f32x2 QB = mul2(mul2(G, fg), bc2(iz));                          // (g0, g1) = (J3, J4)
-#if !AGT_DPR_F32_PROJECTION
-      const f32x2 XY = add2(Yxy, t01);
-#endif
+      const float r = __fsub_rn(I, q.w);
+      const f32x2 QB = mul2(mul2(G, fg), bc2(q.iz));                        // (g0, g1) = (J3, J4)
       const float g0 = lo2(QB), g1 = hi2(QB);
-      const float g2 = -(g0 * lo2(XY) + g1 * hi2(XY)) * iz;
+      const float g2 = __fmul_rn(q.iz, -fmaf(g0, lo2(q.XY), __fmul_rn(g1, hi2(q.XY))));
       // (J0, -J1) = g2 (Yy, Yx) - Yz (g1, g0);  J2 = Yx g1 - Yy g0
-      const f32x2 QA = fma2(bc2(g2), swap2(Yxy), mul2(bc2(-Yz), swap2(QB)));
-      const f32x2 QC = pk2(lo2(Yxy) * g1 - hi2(Yxy) * g0, g2);             // (J2, J5)
+      const f32x2 QA = fma2(bc2(g2), swap2(q.Yxy), mul2(bc2(-q.Yz), swap2(QB)));
+      const f32x2 QC = pk2(fmaf(lo2(q.Yxy), g1, -__fmul_rn(hi2(q.Yxy), g0)), g2);   // (J2, J5)
       const float q0 = lo2(QA), q1 = hi2(QA), q4 = lo2(QC);
       p0 = fma2(bc2(q0), QA, p0); p1 = fma2(bc2(q0), QB, p1); p2 = fma2(bc2(q0), QC, p2);
       p3 = fma2(bc2(q1), QB, p3); p4 = fma2(bc2(q1), QC, p4);
@@ -665,17 +672,40 @@ dpr_kernel(agt_pyramid pyr, agt_camera cam, const float4* __restrict__ samples, 
       scost = fmaf(r, r, scost);
       ++cnt;
     };
-    // This thread's samples are j0, j0 + step, ... of the concatenated active tags.  Software pipeline: the model
-    // record of the next sample is requested before the current one is consumed; two copies of the body alternate
-    // between two record registers so that nothing has to be moved.
+    // One sample by whichever path its footprint needs.
+    auto eval_sample = [&](const DprSample& q) {
+      uint32_t row[4];
+      if (in_tile(q)) {
+        fetch_tile(q, row);
+      } else {
+        const int x0 = q.lx + tx0 + 1, y0 = q.ly + ty0 + 1;
+        // valid <=> z > 1e-6 and 1 <= floor(ul) <= lw-3 and 1 <= floor(vl) <= lh-3
+        if (!q.depth_ok || x0 < 1 || x0 > lw - 3 || y0 < 1 || y0 > lh - 3) return;
+        if (x0 - 1 < S.rx0 || y0 - 1 < S.ry0 || x0 + 3 > S.rx1 || y0 + 3 > S.ry1) S.left_roi = 1;   // benign race: all write 1
+        const uint8_t* g = limg + (int64_t)(y0 - 1) * lpitch + (x0 - 1);
+#pragma unroll
+        for (int r = 0; r < 4; ++r) row[r] = ld4_global(g + r * lpitch);
+      }
+      accumulate(q, row);
+    };
+    // This thread's samples are j0, j0 + step, ... of the concatenated active tags, taken two at a time.  When every lane
+    // of the warp holds two samples whose footprints both lie in the tile (nearly always), the pair runs as one
+    // straight-line body: no branch, no global load, so the two samples' fetches and dp4a chains overlap.  Otherwise
+    // each sample of the pair goes through eval_sample.  Either way a thread adds its samples to its sums in sequence
+    // order.  The model records of the next pair are requested before this pair is consumed.
     const int step = kCluster * DPR_THREADS;
     const int j0 = crank * DPR_THREADS + tid;
+    // (the sample count is read per evaluation: held across the LM phase it is spilled and reloaded ahead of the loop)
+    const int n_act_samples = S.act_prefix[S.n_active];
     int left = j0 < n_act_samples ? (n_act_samples - j0 + step - 1) / step : 0;
-    if (left > 0) {
-      int seg = 0;
-      while (j0 >= S.act_prefix[seg + 1]) ++seg;
-      int sidx = S.act_begin[seg] + (j0 - S.act_prefix[seg]);               // record index of the current sample
-      int seg_last = S.act_begin[seg] + (S.act_prefix[seg + 1] - S.act_prefix[seg]);   // end of this tag's records
+    const int n_pairs = __reduce_max_sync(0xffffffffu, (left + 1) >> 1);      // the lanes of a warp differ by one sample at most
+    if (n_pairs > 0) {
+      int seg = 0, sidx = 0, seg_last = 0;
+      if (left > 0) {
+        while (j0 >= S.act_prefix[seg + 1]) ++seg;
+        sidx = S.act_begin[seg] + (j0 - S.act_prefix[seg]);                   // record index of the current sample
+        seg_last = S.act_begin[seg] + (S.act_prefix[seg + 1] - S.act_prefix[seg]);   // end of this tag's records
+      }
       auto advance = [&]() {
         sidx += step;
         if (sidx >= seg_last) {                        // crossed into the next active tag (rare)
@@ -689,19 +719,25 @@ dpr_kernel(agt_pyramid pyr, agt_camera cam, const float4* __restrict__ samples, 
       // outstanding loads, so a request issued just before the first use of the previous record would make that use
       // wait for the new request as well (seen as 11 % of all stall samples on one instruction).
       const int zero = S.zero;
-      float4 smA = __ldg(&samples[sidx]), smB;
+      float4 smA = make_float4(0.f, 0.f, 1.f, 0.f), smB = smA;                // (a lane without a sample projects a dummy)
+      if (left > 0) smA = __ldg(&samples[sidx]);
+      if (left > 1) { advance(); smB = __ldg(&samples[sidx + (__float_as_int(smA.w) & zero)]); }
 #pragma unroll 1
-      while (true) {
-        const bool moreA = left > 1;
-        if (moreA) advance();
-        smB = __ldg(&samples[sidx + (__float_as_int(smA.w) & zero)]);     // (the last sample re-reads its own record)
-        eval_sample(smA);
-        if (!moreA) break;
-        const bool moreB = left > 2;
-        if (moreB) advance();
-        smA = __ldg(&samples[sidx + (__float_as_int(smB.w) & zero)]);
-        eval_sample(smB);
-        if (!moreB) break;
+      for (int pr = 0; pr < n_pairs; ++pr) {
+        const DprSample qA = project(smA), qB = project(smB);
+        const bool fast = __all_sync(0xffffffffu, left > 1 && in_tile(qA) && in_tile(qB));
+        if (left > 2) { advance(); smA = __ldg(&samples[sidx + (__float_as_int(qA.w) & zero)]); }
+        if (left > 3) { advance(); smB = __ldg(&samples[sidx + (__float_as_int(qB.w) & zero)]); }
+        if (fast) {
+          uint32_t rowA[4], rowB[4];
+          fetch_tile(qA, rowA);
+          fetch_tile(qB, rowB);
+          accumulate(qA, rowA);
+          accumulate(qB, rowB);
+        } else {
+          if (left > 0) eval_sample(qA);
+          if (left > 1) eval_sample(qB);
+        }
         left -= 2;
       }
     }
