@@ -13,12 +13,13 @@
 //   [0] has_prev  [1..6] prev pose  [7] has_guess  [8..13] guess pose
 //   [14] guess arrays alias prev arrays  [15] guess tvec is float32
 //   [16] n_vel  [17..25] rot_vel[0]  [26..28] tran_vel[0]  [29..37] rot_vel[1]  [38..40] tran_vel[1]
+//   [41] prev tvec is float32 (prev holds the arrays of a float32 guess)
 #include "agt_common.cuh"
 
 namespace {
 
 enum { S_HAS_PREV = 0, S_PREV = 1, S_HAS_GUESS = 7, S_GUESS = 8, S_ALIAS = 14, S_T32 = 15, S_NVEL = 16, S_RV0 = 17,
-       S_TV0 = 26, S_RV1 = 29, S_TV1 = 38 };
+       S_TV0 = 26, S_RV1 = 29, S_TV1 = 38, S_P32 = 41 };
 static_assert(S_HAS_GUESS == AGT_STATE_HAS_GUESS && S_GUESS == AGT_STATE_GUESS, "agt_common.cuh: state record slots");
 
 __device__ inline void mat3_mul(const double* A, const double* B, double* C) {      // C = A B
@@ -51,11 +52,12 @@ __device__ inline bool ape_update_stream(double* s, int n_tags, const double* p_
   for (int k = 0; k < 6; ++k) held[k] = s[S_PREV + k];      // deepcopy(prev_transform), detect_pose.py:490
   if (n_tags < 2) { s[S_HAS_GUESS] = 0.0; return false; }   // detect_pose.py:494-496,573-574
   const bool fresh = !(enhance && s[S_HAS_GUESS] != 0.0);
+  const bool t32 = !fresh && s[S_T32] != 0.0;                // the pose lands in float32 tvec arrays
   double p[6];
   for (int k = 0; k < 6; ++k) p[k] = p_in[k];
   if (!fresh) {
     // solvePnP wrote its result into the guess arrays (dtype preserved)
-    if (s[S_T32] != 0.0)
+    if (t32)
       for (int k = 3; k < 6; ++k) p[k] = (double)(float)p[k];
     for (int k = 0; k < 6; ++k) s[S_GUESS + k] = p[k];
     if (s[S_ALIAS] != 0.0)
@@ -71,7 +73,9 @@ __device__ inline bool ape_update_stream(double* s, int n_tags, const double* p_
     double Rp[9], Rcur[9], rv[9], tv[3], dt[3];
     agt_rodrigues(held, Rp);
     agt_rodrigues(p, Rcur);
-    for (int k = 0; k < 3; ++k) dt[k] = held[3 + k] - p[3 + k];
+    // numpy subtracts two float32 tvec arrays in float32 (both are float32 values already: one rounding)
+    const bool f32_sub = t32 && s[S_P32] != 0.0;
+    for (int k = 0; k < 3; ++k) dt[k] = f32_sub ? (double)__fsub_rn((float)held[3 + k], (float)p[3 + k]) : held[3 + k] - p[3 + k];
     mat3_tvec(Rcur, dt, tv);                                 // R_curr^T (t_prev - t_curr)
     mat3_tmul(Rcur, Rp, rv);                                 // R_curr^T R_prev
     bool zero = false;
@@ -121,6 +125,12 @@ __device__ inline bool ape_update_stream(double* s, int n_tags, const double* p_
       for (int r = 0; r < 3; ++r) t2[r] = Ra[r * 3] * t1[0] + Ra[r * 3 + 1] * t1[1] + Ra[r * 3 + 2] * t1[2] + 0.5 * tacc[r];
       double rvec[3];
       agt_log_rotation(R2, rvec);                            // cv.Rodrigues(rmat), detect_pose.py:344
+      // cv::Rodrigues orthonormalises the matrix by an SVD first, which fails on a non-finite matrix: the vector is zero.  The
+      // reference's 4x4 product also makes the rotation non-finite where a translation is (times the next factor's zero row).
+      bool fin = true;
+      for (int k = 0; k < 9; ++k) fin = fin && isfinite(R2[k]);
+      for (int k = 0; k < 3; ++k) fin = fin && isfinite(tacc[k]) && isfinite(tv[k]);
+      if (!fin) rvec[0] = rvec[1] = rvec[2] = 0.0;
       for (int k = 0; k < 3; ++k) s[S_GUESS + k] = rvec[k];
       for (int k = 0; k < 3; ++k) s[S_GUESS + 3 + k] = (double)(float)t2[k];   // transform_helper.py:158-159
       s[S_HAS_GUESS] = 1.0; s[S_ALIAS] = 0.0; s[S_T32] = 1.0;
@@ -130,6 +140,7 @@ __device__ inline bool ape_update_stream(double* s, int n_tags, const double* p_
   }
   for (int k = 0; k < 6; ++k) s[S_PREV + k] = p[k];          // detect_pose.py:569
   s[S_HAS_PREV] = 1.0;
+  s[S_P32] = t32 ? 1.0 : 0.0;
   return true;
 }
 

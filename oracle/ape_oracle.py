@@ -19,9 +19,10 @@ cv2.solvePnP with useExtrinsicGuess=True writes its result INTO the guess
 arrays (dtype preserved, so a float32 tvec guess yields a float32-rounded
 tvec); ``extrinsic_guess`` aliases ``prev_transform`` after the first accepted
 frame (detect_pose.py:551,569); the predictor composes the inverse-motion
-"velocities" onto the previous pose (detect_pose.py:341); velocity buffers are
-not cleared on tracking loss; exact zeros in a velocity raise ValueError
-(detect_pose.py:236-237).
+"velocities" onto the previous pose (detect_pose.py:341); two float32 tvec
+arrays are subtracted in float32; velocity buffers are not cleared on tracking
+loss; exact zeros in a velocity raise ValueError (detect_pose.py:236-237), which
+``step_given`` reports as an error flag.
 """
 from __future__ import annotations
 
@@ -105,6 +106,7 @@ class ApeOracle:
         self.tran_vel: List[np.ndarray] = []
         self.last_error = None      # mean reprojection error of the last solved frame
         self.last_accepted = False
+        self.last_t64 = None
 
     # -- predictor --------------------------------------------------------
     def _velocities(self, curr, prev):
@@ -131,42 +133,93 @@ class ApeOracle:
         rmat = cv.Rodrigues(base[0])[0]
         pred = _homogeneous(half, 0.5 * tacc) @ _homogeneous(rot, tran) @ _homogeneous(rmat, base[1])  # :334-341
         r_out = pred[0:3, 0:3]
+        self.last_t64 = pred[0:3, 3].copy()                               # the predicted tvec before its float32 rounding
         t_out = np.array(pred[0:3, 3], dtype=np.float32).reshape(3, -1)  # transform_helper.py:158-159
         return cv.Rodrigues(r_out)[0], t_out
 
     # -- one frame ----------------------------------------------------------
     def step(self, dets: Sequence[Tuple[int, np.ndarray]]):
-        """dets: accepted detections [(tag_id, corners (4,2))].  Mutates the state."""
-        held_prev = copy.deepcopy(self.prev)              # detect_pose.py:490
+        """dets: accepted detections [(tag_id, corners (4,2))].  Mutates the state: solvePnP and the mean reprojection
+        error (detect_pose.py:494-538), then ``step_given``."""
         self.last_error = None
-        self.last_accepted = False
         if len(dets) < MIN_TAGS:
-            self.guess = (None, None)                     # detect_pose.py:573-574
-            return
+            return self.step_given(len(dets), None, False, None)
         obj = np.array([tag_object_points(*self._sz_r_t(t)) for t, _ in dets], dtype=np.float32).reshape(-1, 3)
         img = np.array([np.asarray(c).reshape(1, 4, 2) for _, c in dets], dtype=np.float32).reshape(-1, 2)
-        fresh = self.guess[0] is None or not self.enhance_ape
-        if fresh:
+        if self.guess[0] is None or not self.enhance_ape:
             ok, rvec, tvec = cv.solvePnP(obj, img, self.mtx, self.dist, flags=cv.SOLVEPNP_ITERATIVE)
         else:
-            ok, rvec, tvec = cv.solvePnP(obj, img, self.mtx, self.dist, self.guess[0], self.guess[1], True,
+            # (on copies of the guess arrays: step_given makes solvePnP's write into them, after it holds prev)
+            ok, rvec, tvec = cv.solvePnP(obj, img, self.mtx, self.dist, self.guess[0].copy(), self.guess[1].copy(), True,
                                          flags=cv.SOLVEPNP_ITERATIVE)
-        pose = (rvec, tvec)
+        err = None
+        if ok:
+            err = mean_reprojection_error(obj, img, rvec, tvec, self.mtx, self.dist)
+            self.last_error = float(err)
+        return self.step_given(len(dets), (rvec, tvec), ok, err)
+
+    def step_given(self, n_tags: int, pose, ok: bool, err) -> bool:
+        """detect_pose.py:490-574 applied to a pose it is handed (what solvePnP, or the dense refinement, returned):
+        n_tags accepted detections, pose (rvec, tvec) or 6 values, ok, err the mean reprojection error.  Mutates the
+        state; sets ``last_accepted`` and returns the error flag: True where the reference raises ValueError on a
+        zero entry in a velocity (detect_pose.py:236-237).  The state is then left as the reference held it when it
+        raised: the guess arrays already overwritten, the velocities not appended, prev touched only through the
+        aliased guess arrays; ``last_accepted`` is True (the pose passed the gate)."""
+        held_prev = copy.deepcopy(self.prev)              # detect_pose.py:490
+        self.last_accepted = False
+        self.last_t64 = None
+        if n_tags < MIN_TAGS:
+            self.guess = (None, None)                     # detect_pose.py:573-574
+            return False
+        fresh = self.guess[0] is None or not self.enhance_ape
+        if pose is not None and not isinstance(pose, tuple):
+            pose = (np.asarray(pose, dtype=np.float64).reshape(6)[:3], np.asarray(pose, dtype=np.float64).reshape(6)[3:])
+        if fresh:
+            pose = (np.array(pose[0], dtype=np.float64).reshape(3, 1), np.array(pose[1], dtype=np.float64).reshape(3, 1))
+        else:
+            # solvePnP(useExtrinsicGuess=True) writes its result into the guess arrays, dtype preserved (a float32 tvec
+            # after a prediction), and returns them; they are prev_transform's arrays too after a fresh solve
+            self.guess[0][...] = np.asarray(pose[0]).reshape(self.guess[0].shape)
+            self.guess[1][...] = np.asarray(pose[1]).reshape(self.guess[1].shape)
+            pose = self.guess
         if not ok:
-            return                                         # detect_pose.py:533 (no else branch: state untouched)
-        err = mean_reprojection_error(obj, img, rvec, tvec, self.mtx, self.dist)
-        self.last_error = float(err)
+            return False                                   # detect_pose.py:533 (no else branch: state untouched)
         if not err < MAX_MEAN_ERROR:
             self.guess = (None, None)                      # detect_pose.py:570-572
-            return
+            return False
         self.last_accepted = True
         if fresh:
             self.guess = pose                              # detect_pose.py:551
         else:
-            good, tran, rot, tacc, racc = self._velocities(pose, held_prev)
+            try:
+                good, tran, rot, tacc, racc = self._velocities(pose, held_prev)
+            except ValueError:
+                return True
             if good:
                 self.guess = self._predict(held_prev, tran, tacc, rot, racc)   # detect_pose.py:558-566
         self.prev = pose                                   # detect_pose.py:569
+        return False
+
+    def state_record(self) -> np.ndarray:
+        """The state as the device keeps it (AGT_STREAM_STATE_DOUBLES doubles, layout at the top of csrc/agt_ape.cu):
+        has_prev, prev, has_guess, guess, guess aliases prev, guess tvec is float32, n_vel, rot/tran velocity slots
+        (oldest first), prev tvec is float32 (slot 41), zeros beyond.  Without a guess its slots 8-15 are 0 (the device leaves them stale)."""
+        s = np.zeros(64)
+        if self.prev[0] is not None:
+            s[0] = 1.0
+            s[1:4], s[4:7] = np.ravel(self.prev[0]), np.ravel(self.prev[1])
+        if self.guess[0] is not None:
+            s[7] = 1.0
+            s[8:11], s[11:14] = np.ravel(self.guess[0]), np.ravel(self.guess[1])
+            s[14] = float(self.guess[0] is self.prev[0] and self.guess[1] is self.prev[1])
+            s[15] = float(np.asarray(self.guess[1]).dtype == np.float32)
+        if self.prev[0] is not None:
+            s[41] = float(np.asarray(self.prev[1]).dtype == np.float32)
+        s[16] = len(self.rot_vel)
+        for k, (rot, tran) in enumerate(zip(self.rot_vel, self.tran_vel)):
+            s[17 + 12 * k:26 + 12 * k] = np.ravel(rot)
+            s[26 + 12 * k:29 + 12 * k] = np.ravel(tran)
+        return s
 
     def _sz_r_t(self, tag_id):
         size, tvec, rvec = self.group[tag_id]

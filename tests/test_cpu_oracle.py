@@ -36,6 +36,55 @@ def test_ape_oracle_reproduces_reference_golden_bit_exact():
     assert lost == [30, 31, 50]
 
 
+def test_ape_oracle_state_record_follows_the_golden_sequence():
+    """state_record() (the device's layout) carries the same prev / guess / n_vel as the snapshots of the golden run."""
+    g = np.load(GOLDEN / "ape_sequence.npz")
+    orc = ape_oracle.ApeOracle(ape_oracle.group_from_json(synth.april_group_dict()), g["mtx"], None, True)
+    for f in range(g["ids"].shape[0]):
+        orc.step(make_golden.unpack_detections(g["ids"], g["corners"], f))
+        s = orc.state_record()
+        assert s.shape == (64,) and not s[42:].any()
+        assert s[0] == (not np.isnan(g["prev"][f][0])) and s[7] == (not np.isnan(g["guess"][f][0])) and s[16] == g["n_vel"][f]
+        if s[0]:
+            assert np.array_equal(s[1:7], g["prev"][f])
+        if s[7]:
+            assert np.array_equal(s[8:14], g["guess"][f])
+            assert s[15] == (orc.last_t64 is not None)    # a float32 tvec exactly when the guess is a prediction
+            assert s[14] == (orc.last_t64 is None)        # otherwise the guess arrays are prev's
+
+
+def test_ape_oracle_step_given_models_the_guess_write_and_the_raise():
+    """step_given on poses it is handed: the write of solvePnP into the (aliased, float32) guess arrays, and the state the
+    reference is left in when a zero velocity raises."""
+    rng = np.random.default_rng(4)
+    orc = ape_oracle.ApeOracle(ape_oracle.group_from_json(synth.april_group_dict()), synth.CAMERA_VGA.mtx, None, True)
+    poses = [np.concatenate([rng.normal(0, 0.5, 3), [0.01 * k, -0.02, 0.4 + 0.01 * k * k]]) for k in range(5)]
+    assert not orc.step_given(3, poses[0], True, 0.5)
+    s = orc.state_record()
+    assert s[0] == s[7] == s[14] == 1 and s[15] == 0 and np.array_equal(s[1:7], poses[0]) and np.array_equal(s[8:14], poses[0])
+    # the same pose again: a zero translation velocity raises in the reference -> error flag, nothing appended
+    assert orc.step_given(3, poses[0], True, 0.5) and orc.last_accepted and orc.state_record()[16] == 0
+    # PnP fails: its zeros land in the guess arrays and, aliased, in prev
+    assert not orc.step_given(3, np.zeros(6), False, 0.0) and not orc.last_accepted
+    s = orc.state_record()
+    assert not s[1:7].any() and not s[8:14].any() and s[14] == 1
+    for k in (1, 2, 3):
+        assert not orc.step_given(3, poses[k], True, 0.5)
+    s = orc.state_record()
+    assert s[16] == 2 and s[14] == 0 and s[15] == 1 and orc.guess[1].dtype == np.float32
+    # (the pose of the frame after the prediction came through the float32 guess arrays)
+    assert np.array_equal(s[1:4], poses[3][:3]) and np.array_equal(s[4:7], poses[3][3:].astype(np.float32))
+    # with a float32 guess, the pose handed in is rounded on its way into it; prev (not aliased) keeps its value
+    assert not orc.step_given(3, poses[4], False, 0.0)
+    s = orc.state_record()
+    assert np.array_equal(s[11:14], poses[4][3:].astype(np.float32)) and np.array_equal(s[8:11], poses[4][:3])
+    assert np.array_equal(s[1:4], poses[3][:3]) and np.array_equal(s[4:7], poses[3][3:].astype(np.float32))
+    # fewer than two tags drop the guess; the velocities stay
+    assert not orc.step_given(1, poses[4], True, 0.5)
+    s = orc.state_record()
+    assert s[7] == 0 and not s[8:16].any() and s[16] == 2
+
+
 def test_object_points_match_reference_golden():
     g = np.load(GOLDEN / "ape_sequence.npz")
     assert np.allclose(synth.object_points(), g["all_objpts"], atol=1e-9)
