@@ -139,7 +139,6 @@ extern "C" int agt_destroy(agt_ctx* ctx) {
   if (ctx->d_remap_tab) cudaFree(ctx->d_remap_tab);
   if (ctx->d_tag_codes) cudaFree(ctx->d_tag_codes);
   if (ctx->h_rects) cudaFreeHost(ctx->h_rects);
-  if (ctx->h_prects) cudaFreeHost(ctx->h_prects);
   for (int k = 0; k < 2; ++k) { if (ctx->h_stage[k]) cudaFreeHost(ctx->h_stage[k]); if (ctx->ev_stage[k]) cudaEventDestroy(ctx->ev_stage[k]); }
   for (int i = 0; i < 4; ++i) if (ctx->ev[i]) cudaEventDestroy(ctx->ev[i]);
   cudaStreamDestroy(ctx->own_stream);
@@ -442,14 +441,6 @@ extern "C" int agt_set_upload_threads(agt_ctx* ctx, int threads) {
   return AGT_OK;
 }
 
-static bool roi_rect_l0(const agt_ctx* ctx, const agt_pyramid& one, const double* init, int n_hyp, int* X0, int* Y0, int* X1,
-                        int* Y1) {
-  int32_t r[4];
-  bool ok = agt_dpr_rect_l0(ctx->cam, ctx->model.pitch, ctx->model.radius, init, n_hyp, one.width, one.height, one.levels, r);
-  *X0 = r[0]; *Y0 = r[1]; *X1 = r[2]; *Y1 = r[3];
-  return ok;
-}
-
 extern "C" int agt_set_roi_upload(agt_ctx* ctx, int enable) {
   if (!ctx) return AGT_ERR_INVALID;
   ctx->roi_upload = enable ? 1 : 0;
@@ -458,104 +449,174 @@ extern "C" int agt_set_roi_upload(agt_ctx* ctx, int enable) {
 
 extern "C" int64_t agt_last_h2d_bytes(const agt_ctx* ctx) { return ctx ? ctx->last_h2d_bytes : -1; }
 
-// One pass of chunked, double-buffered refinement over the frames listed in `ids` (NULL = 0..count-1).
-// roi != 0 uploads only the rectangle each refinement can touch.
-static int refine_pass(agt_ctx* ctx, const uint8_t* h_frames, int w, int h, int levels, const int* ids, int count,
-                       int n_hyp, int roi, const double* h_init, uint8_t* dr, size_t o_init, size_t o_pose, size_t o_cost,
-                       size_t o_nv, size_t o_ev, size_t o_st, size_t o_left, int chunk, uint8_t* const buf[2]) {
+// scratch slots of agt_refine_host (slot 5 holds the job records of refine_impl in agt_dpr.cu)
+constexpr int SLOT_CHUNK0 = 0, SLOT_CHUNK1 = 1, SLOT_JOBS = 2, SLOT_REDO_JOBS = 3, SLOT_RECTS = 4, SLOT_STAGE = 6;
+
+// The per-job arrays of one refinement pass (init and pose: 6 doubles per job; left: the refinement read outside the
+// rectangle its frame was given).
+struct agt_jobs { double *init, *pose; float* cost; int32_t *n_valid, *evals; uint8_t *status, *left; };
+
+// Lay the arrays of `jobs` jobs out back to back from `base` (nullptr: size only); returns their bytes.
+static size_t layout_jobs(agt_jobs* a, uint8_t* base, int64_t jobs) {
+  size_t off = 0;
+  auto next = [&](size_t per_job) { uint8_t* p = base ? base + off : nullptr; off += align_up(per_job * jobs, 256); return p; };
+  a->init = reinterpret_cast<double*>(next(sizeof(double) * 6));
+  a->pose = reinterpret_cast<double*>(next(sizeof(double) * 6));
+  a->cost = reinterpret_cast<float*>(next(sizeof(float)));
+  a->n_valid = reinterpret_cast<int32_t*>(next(sizeof(int32_t)));
+  a->evals = reinterpret_cast<int32_t*>(next(sizeof(int32_t)));
+  a->status = next(1);
+  a->left = next(1);
+  return off;
+}
+
+// Grow `n` page-locked host buffers of `*bytes` each to at least `need` bytes.  They are kept across calls: page-locking
+// memory in every call would add its cost to every call.
+static int grow_pinned(agt_ctx* ctx, uint8_t** bufs, int n, size_t* bytes, size_t need) {
+  if (*bytes >= need) return AGT_OK;
+  for (int k = 0; k < n; ++k) { if (bufs[k]) cudaFreeHost(bufs[k]); bufs[k] = nullptr; }
+  *bytes = 0;
+  for (int k = 0; k < n; ++k) AGT_CUDA(ctx, cudaMallocHost(reinterpret_cast<void**>(&bufs[k]), need));
+  *bytes = need;
+  return AGT_OK;
+}
+
+static int64_t rect_area(const agt_roi_rect& r) { return (int64_t)(r.x1 - r.x0) * (r.y1 - r.y0); }
+
+// ROI pass: only each frame's rectangle reaches the device, and the refinement builds the part of its pyramid level it
+// reads itself (K1 fused into K4).  WHOLE (ROI upload off) and REDO (the frames whose ROI refinement left its rectangle):
+// whole frames, full pyramid, plain refinement - the result then cannot depend on any ROI prediction.
+enum pass_kind { PASS_ROI, PASS_WHOLE, PASS_REDO };
+
+struct refine_pass_desc {
+  pass_kind kind;
+  const uint8_t* frames;             // host frames, w x h bytes each
+  const uint8_t* frames_dev;         // their device alias (pinned, device-mapped memory) or nullptr
+  const double* init;                // host initial poses [frame][n_hyp][6] the ROI pass derives the rectangles from
+  int w, h, levels, n_hyp, chunk;
+  std::vector<agt_roi_rect> rects;   // per frame of the pass: the level-0 rectangle to upload (empty: none) and its host frame
+};
+
+// How the frames of a pass reach the chunk buffers:
+//   GATHER  one roi_gather_kernel launch per chunk reads the rectangles out of pinned, device-mapped frames
+//   STAGED  host threads pack a chunk's rectangles of pageable frames into pinned staging, one copy, one roi_scatter_kernel
+//   WHOLE   one copy per chunk of contiguous whole frames
+//   COPIES  one cudaMemcpy2DAsync per rectangle
+enum upload_path { UPLOAD_GATHER, UPLOAD_STAGED, UPLOAD_WHOLE, UPLOAD_COPIES };
+
+// One pass of chunked, double-buffered refinement: the H2D of chunk c+1 on the copy stream overlaps the refinement of
+// chunk c.  Jobs of chunk c are contiguous in J: [b0*n_hyp, (b0+nb)*n_hyp).
+static int refine_pass(agt_ctx* ctx, refine_pass_desc& d, const agt_jobs& J, uint8_t* const buf[2]) {
   cudaStream_t st = ctx->stream, cp = ctx->copy_stream;
+  const int count = (int)d.rects.size(), w = d.w, h = d.h;
+  // The ROI pass computes its rectangles chunk by chunk, right before the chunk's upload: the CPU work of chunk c+1 then
+  // runs while chunk c is copied and refined.  STAGED sizes its staging from all of them, so it computes them up front.
   agt_pyramid one;
-  layout_pyramid(&one, nullptr, w, h, levels, 1);
-  const bool tight = one.pitch[0] == w;
+  layout_pyramid(&one, nullptr, w, h, d.levels, 1);
+  int filled = d.kind == PASS_ROI ? 0 : count;
+  auto fill_rects = [&](int end) {
+    for (int32_t q[4]; filled < end; ++filled) {
+      agt_dpr_rect_l0(ctx->cam, ctx->model.pitch, ctx->model.radius, d.init + (int64_t)filled * d.n_hyp * 6, d.n_hyp, one.width,
+                      one.height, one.levels, q);
+      d.rects[(size_t)filled] = {q[0], q[1], q[2], q[3], filled};
+    }
+  };
+  // the upload path of this pass (the kernels move 16-byte row pieces; WHOLE needs level 0 at pitch w), and what it
+  // needs, set up here and nowhere else
+  const bool roi16 = d.kind == PASS_ROI && (w & 15) == 0;
+  upload_path path = d.kind == PASS_WHOLE && (w & 15) == 0 ? UPLOAD_WHOLE : UPLOAD_COPIES;
+  if (roi16 && d.frames_dev && (reinterpret_cast<uintptr_t>(d.frames_dev) & 15) == 0) path = UPLOAD_GATHER;
+  if (roi16 && !d.frames_dev && ctx->upload_threads > 0) path = UPLOAD_STAGED;
   int rc;
-  int n_chunks = (count + chunk - 1) / chunk;
-  for (int c = 0; c < n_chunks; ++c) {
-    int b0 = c * chunk, nb = count - b0 < chunk ? count - b0 : chunk;
-    int s = c & 1;
+  void* d_rects = nullptr;
+  uint8_t* d_stage = nullptr;
+  if (path == UPLOAD_GATHER || path == UPLOAD_STAGED) {
+    // one pinned list slot per frame of the pass, so the CPU never overwrites a list whose asynchronous upload is pending
+    const size_t list_bytes = (path == UPLOAD_GATHER ? sizeof(agt_roi_rect) : sizeof(agt_pack_rect)) * (size_t)count;
+    if ((rc = grow_pinned(ctx, &ctx->h_rects, 1, &ctx->rect_bytes, list_bytes))) return rc;
+    if ((rc = agt_scratch(ctx, SLOT_RECTS, list_bytes, &d_rects))) return rc;
+  }
+  if (path == UPLOAD_STAGED) {
+    // staging: 2 x the largest chunk's rectangles, on the host and on the device
+    fill_rects(count);
+    int64_t need = 0;
+    for (int b0 = 0; b0 < count; b0 += d.chunk) {
+      int64_t sum = 0;
+      for (int i = b0; i < count && i < b0 + d.chunk; ++i) sum += rect_area(d.rects[(size_t)i]);
+      need = sum > need ? sum : need;
+    }
+    if ((rc = grow_pinned(ctx, ctx->h_stage, 2, &ctx->stage_bytes, (size_t)align_up(need + 256, 4096)))) return rc;
+    if ((rc = agt_scratch(ctx, SLOT_STAGE, 2 * ctx->stage_bytes, reinterpret_cast<void**>(&d_stage)))) return rc;
+    for (int k = 0; k < 2; ++k)
+      if (!ctx->ev_stage[k]) AGT_CUDA(ctx, cudaEventCreateWithFlags(&ctx->ev_stage[k], cudaEventDisableTiming));
+  }
+  for (int c = 0, b0 = 0; b0 < count; ++c, b0 += d.chunk) {
+    const int nb = count - b0 < d.chunk ? count - b0 : d.chunk, s = c & 1;
+    const agt_roi_rect* r = d.rects.data() + b0;
     agt_pyramid p;
-    layout_pyramid(&p, buf[s], w, h, levels, chunk);
+    layout_pyramid(&p, buf[s], w, h, d.levels, d.chunk);
     if (c >= 2) AGT_CUDA(ctx, cudaStreamWaitEvent(cp, ctx->ev[s], 0));       // compute on this buffer finished
-    const bool contiguous_ids = ids == nullptr;
-    if (roi && ctx->host_frames_dev && (w & 15) == 0 && (reinterpret_cast<uintptr_t>(ctx->host_frames_dev) & 15) == 0) {
-      // rectangles of this chunk -> device, then one gather launch on the copy stream
-      agt_roi_rect* hr = ctx->h_rects + b0;        // pinned; one slot per frame of the pass, so the CPU never
-      agt_roi_rect* drc = ctx->d_rects + b0;       // overwrites a list whose asynchronous upload is still pending
-      for (int i = 0; i < nb; ++i) {
-        int f = ids ? ids[b0 + i] : b0 + i;
-        agt_roi_rect r = {0, 0, 0, 0, f};
-        if (roi_rect_l0(ctx, one, h_init + (int64_t)f * n_hyp * 6, n_hyp, &r.x0, &r.y0, &r.x1, &r.y1))
-          ctx->last_h2d_bytes += (int64_t)(r.x1 - r.x0) * (r.y1 - r.y0);
-        else
-          r.x0 = r.x1 = r.y0 = r.y1 = 0;
-        hr[i] = r;
-      }
+    fill_rects(b0 + nb);
+    int64_t bytes = 0;
+    for (int i = 0; i < nb; ++i) bytes += rect_area(r[i]);
+    if (path == UPLOAD_GATHER) {
+      agt_roi_rect* hr = reinterpret_cast<agt_roi_rect*>(ctx->h_rects) + b0;
+      agt_roi_rect* drc = static_cast<agt_roi_rect*>(d_rects) + b0;
+      memcpy(hr, r, sizeof(agt_roi_rect) * nb);
       AGT_CUDA(ctx, cudaMemcpyAsync(drc, hr, sizeof(agt_roi_rect) * nb, cudaMemcpyHostToDevice, cp));
       // 64 CTAs: enough 16-byte reads in flight to fill PCIe, few enough to leave the SMs to the compute stream
       // (measured 32 / 64 / 128 / 256 CTAs x chunk 128..1024 frames: profiles/r01_e2e_sweep.log)
-      roi_gather_kernel<<<nb < 64 ? nb : 64, 256, 0, cp>>>(ctx->host_frames_dev, w, h, drc, p.data[0], p.pitch[0], p.frame_stride[0], nb);
+      roi_gather_kernel<<<nb < 64 ? nb : 64, 256, 0, cp>>>(d.frames_dev, w, h, drc, p.data[0], p.pitch[0], p.frame_stride[0], nb);
       AGT_LAUNCH_CHECK(ctx);
-    } else if (!roi && contiguous_ids && tight) {
-      AGT_CUDA(ctx, cudaMemcpyAsync(p.data[0], h_frames + (int64_t)b0 * w * h, (size_t)nb * w * h, cudaMemcpyHostToDevice, cp));
-      ctx->last_h2d_bytes += (int64_t)nb * w * h;
-    } else if (roi && ctx->upload_threads > 0 && (w & 15) == 0 && ctx->h_stage[0] != nullptr) {
-      // pageable frames: pack the chunk's ROI rows into pinned staging with a few threads, one copy, one scatter launch
-      agt_pack_rect* hr = ctx->h_prects + b0;
+    } else if (path == UPLOAD_STAGED) {
+      agt_pack_rect* hr = reinterpret_cast<agt_pack_rect*>(ctx->h_rects) + b0;
       std::vector<int> src_frame((size_t)nb);
       long long off = 0;
       for (int i = 0; i < nb; ++i) {
-        int f = ids ? ids[b0 + i] : b0 + i;
-        src_frame[(size_t)i] = f;
-        agt_pack_rect r = {0, 0, 0, 0, off};
-        if (!roi_rect_l0(ctx, one, h_init + (int64_t)f * n_hyp * 6, n_hyp, &r.x0, &r.y0, &r.x1, &r.y1)) r.x0 = r.x1 = r.y0 = r.y1 = 0;
-        off += (long long)(r.x1 - r.x0) * (r.y1 - r.y0);
-        hr[i] = r;
+        src_frame[(size_t)i] = r[i].src;
+        hr[i] = {r[i].x0, r[i].y0, r[i].x1, r[i].y1, off};
+        off += rect_area(r[i]);
       }
-      if ((size_t)off > ctx->stage_bytes)
-        AGT_FAIL(ctx, AGT_ERR_INVALID, "agt_refine_host: ROI rectangles of a chunk (%lld bytes) exceed the staging buffer", off);
       // the staging buffer of this parity was last read by the copy of chunk c-2
       if (c >= 2) AGT_CUDA(ctx, cudaEventSynchronize(ctx->ev_stage[s]));
-      {
-        const int nt = ctx->upload_threads < nb ? ctx->upload_threads : nb;
-        std::vector<std::thread> pool;
-        for (int t = 1; t < nt; ++t)
-          pool.emplace_back(pack_rows, h_frames, w, h, src_frame.data(), hr, (int)((int64_t)nb * t / nt), (int)((int64_t)nb * (t + 1) / nt),
-                            ctx->h_stage[s]);
-        pack_rows(h_frames, w, h, src_frame.data(), hr, 0, (int)((int64_t)nb / nt), ctx->h_stage[s]);
-        for (auto& th : pool) th.join();
-      }
-      uint8_t* dpk = ctx->d_stage + (size_t)s * ctx->stage_bytes;
+      const int nt = ctx->upload_threads < nb ? ctx->upload_threads : nb;
+      auto pack = [&](int t) {
+        pack_rows(d.frames, w, h, src_frame.data(), hr, (int)((int64_t)nb * t / nt), (int)((int64_t)nb * (t + 1) / nt), ctx->h_stage[s]);
+      };
+      std::vector<std::thread> pool;
+      int t = 1;
+      try {
+        for (; t < nt; ++t) pool.emplace_back(pack, t);
+      } catch (const std::exception&) {}        // slice t found no thread: this thread packs t.. itself (the same bytes)
+      pack(0);
+      for (int u = t; u < nt; ++u) pack(u);
+      for (auto& th : pool) th.join();
+      uint8_t* dpk = d_stage + (size_t)s * ctx->stage_bytes;
+      agt_pack_rect* drc = static_cast<agt_pack_rect*>(d_rects) + b0;
       AGT_CUDA(ctx, cudaMemcpyAsync(dpk, ctx->h_stage[s], (size_t)off, cudaMemcpyHostToDevice, cp));
       AGT_CUDA(ctx, cudaEventRecord(ctx->ev_stage[s], cp));
-      AGT_CUDA(ctx, cudaMemcpyAsync(ctx->d_prects + b0, hr, sizeof(agt_pack_rect) * nb, cudaMemcpyHostToDevice, cp));
-      roi_scatter_kernel<<<nb < 296 ? nb : 296, 256, 0, cp>>>(dpk, ctx->d_prects + b0, p.data[0], p.pitch[0], p.frame_stride[0], nb);
+      AGT_CUDA(ctx, cudaMemcpyAsync(drc, hr, sizeof(agt_pack_rect) * nb, cudaMemcpyHostToDevice, cp));
+      roi_scatter_kernel<<<nb < 296 ? nb : 296, 256, 0, cp>>>(dpk, drc, p.data[0], p.pitch[0], p.frame_stride[0], nb);
       AGT_LAUNCH_CHECK(ctx);
-      ctx->last_h2d_bytes += off;
+    } else if (path == UPLOAD_WHOLE) {
+      AGT_CUDA(ctx, cudaMemcpyAsync(p.data[0], d.frames + (int64_t)b0 * w * h, (size_t)nb * w * h, cudaMemcpyHostToDevice, cp));
     } else {
       for (int i = 0; i < nb; ++i) {
-        int f = ids ? ids[b0 + i] : b0 + i;
-        const uint8_t* src = h_frames + (int64_t)f * w * h;
-        uint8_t* dst = p.data[0] + (int64_t)i * p.frame_stride[0];
-        int X0 = 0, Y0 = 0, X1 = w, Y1 = h;
-        if (roi && !roi_rect_l0(ctx, one, h_init + (int64_t)f * n_hyp * 6, n_hyp, &X0, &Y0, &X1, &Y1)) continue;
-        AGT_CUDA(ctx, cudaMemcpy2DAsync(dst + (int64_t)Y0 * p.pitch[0] + X0, (size_t)p.pitch[0], src + (int64_t)Y0 * w + X0, (size_t)w,
-                                        (size_t)(X1 - X0), (size_t)(Y1 - Y0), cudaMemcpyHostToDevice, cp));
-        ctx->last_h2d_bytes += (int64_t)(X1 - X0) * (Y1 - Y0);
+        if (rect_area(r[i]) == 0) continue;
+        const agt_roi_rect& q = r[i];
+        AGT_CUDA(ctx, cudaMemcpy2DAsync(p.data[0] + (int64_t)i * p.frame_stride[0] + (int64_t)q.y0 * p.pitch[0] + q.x0, (size_t)p.pitch[0],
+                                        d.frames + (int64_t)q.src * w * h + (int64_t)q.y0 * w + q.x0, (size_t)w,
+                                        (size_t)(q.x1 - q.x0), (size_t)(q.y1 - q.y0), cudaMemcpyHostToDevice, cp));
       }
     }
+    ctx->last_h2d_bytes += bytes;
     AGT_CUDA(ctx, cudaEventRecord(ctx->ev[2], cp));
     AGT_CUDA(ctx, cudaStreamWaitEvent(st, ctx->ev[2], 0));
-    // ROI pass: only the rectangle of level 0 each refinement can read is on the device, and the refinement builds
-    // the part of its pyramid level it needs itself (K1 fused into K4).  Redo pass (roi == 0): whole frames, full
-    // pyramid, plain refinement - the result then cannot depend on any ROI prediction.
-    if (!roi) {
-      if ((rc = agt_build_pyramid(ctx, &p, nb))) return rc;
-    }
-    // jobs of this chunk are contiguous in the compacted device arrays [b0*n_hyp, (b0+nb)*n_hyp)
-    int64_t j0 = (int64_t)b0 * n_hyp;
-    if ((rc = (roi ? agt_refine_fused : agt_refine)(ctx, &p, reinterpret_cast<double*>(dr + o_init) + j0 * 6, n_hyp, nullptr,
-                         reinterpret_cast<double*>(dr + o_pose) + j0 * 6, reinterpret_cast<float*>(dr + o_cost) + j0,
-                         reinterpret_cast<int32_t*>(dr + o_nv) + j0, reinterpret_cast<int32_t*>(dr + o_ev) + j0,
-                         dr + o_st + j0, dr + o_left + j0, nb)))
+    if (d.kind != PASS_ROI && (rc = agt_build_pyramid(ctx, &p, nb))) return rc;
+    const int64_t j0 = (int64_t)b0 * d.n_hyp;
+    if ((rc = (d.kind == PASS_ROI ? agt_refine_fused : agt_refine)(ctx, &p, J.init + j0 * 6, d.n_hyp, nullptr, J.pose + j0 * 6,
+                                                                   J.cost + j0, J.n_valid + j0, J.evals + j0, J.status + j0,
+                                                                   J.left + j0, nb)))
       return rc;
     AGT_CUDA(ctx, cudaEventRecord(ctx->ev[s], st));
   }
@@ -564,7 +625,7 @@ static int refine_pass(agt_ctx* ctx, const uint8_t* h_frames, int w, int h, int 
 
 extern "C" int agt_refine_host(agt_ctx* ctx, const uint8_t* h_frames, int w, int h, int levels, int batch,
                                const double* h_init, int n_hyp, double* h_pose, float* h_cost, int32_t* h_n_valid,
-                               int32_t* h_evals, uint8_t* h_status, int32_t* h_best) {
+                               int32_t* h_evals, uint8_t* h_status, int32_t* h_best) try {
   if (!ctx) return AGT_ERR_INVALID;
   if (!ctx->camera_set || !ctx->model_set) AGT_FAIL(ctx, AGT_ERR_NOT_READY, "agt_refine_host: camera and surface model must be set");
   if (!h_frames || !h_init || !h_pose || w < 1 || h < 1 || levels < 1 || levels > AGT_MAX_LEVELS || batch < 0 || n_hyp < 1)
@@ -575,7 +636,6 @@ extern "C" int agt_refine_host(agt_ctx* ctx, const uint8_t* h_frames, int w, int
   const bool trace = getenv("AGT_TRACE") != nullptr;      // debug aid: phase timestamps on stderr
   auto t_start = std::chrono::steady_clock::now();
   auto since = [&]() { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_start).count(); };
-  // chunked, double-buffered: H2D of chunk i+1 on the copy stream overlaps pyramid + refinement of chunk i
   agt_pyramid one;
   int64_t per_frame = layout_pyramid(&one, nullptr, w, h, levels, 1);
   // chunks of up to 1024 frames (<= 3 GiB per buffer): large enough that one refinement launch fills the GPU
@@ -586,136 +646,89 @@ extern "C" int agt_refine_host(agt_ctx* ctx, const uint8_t* h_frames, int w, int
   int64_t chunk_bytes = layout_pyramid(&one, nullptr, w, h, levels, chunk);
   uint8_t* buf[2];
   int rc;
-  if ((rc = agt_scratch(ctx, 0, (size_t)chunk_bytes, reinterpret_cast<void**>(&buf[0])))) return rc;
-  if ((rc = agt_scratch(ctx, 1, (size_t)chunk_bytes, reinterpret_cast<void**>(&buf[1])))) return rc;
-  int64_t jobs = (int64_t)batch * n_hyp;
+  if ((rc = agt_scratch(ctx, SLOT_CHUNK0, (size_t)chunk_bytes, reinterpret_cast<void**>(&buf[0])))) return rc;
+  if ((rc = agt_scratch(ctx, SLOT_CHUNK1, (size_t)chunk_bytes, reinterpret_cast<void**>(&buf[1])))) return rc;
+  const int64_t jobs = (int64_t)batch * n_hyp;
+  agt_jobs J;
+  const size_t jobs_bytes = layout_jobs(&J, nullptr, jobs);
   uint8_t* dr;
-  size_t o_init = 0, o_pose = o_init + align_up(sizeof(double) * 6 * jobs, 256), o_cost = o_pose + align_up(sizeof(double) * 6 * jobs, 256),
-         o_nv = o_cost + align_up(sizeof(float) * jobs, 256), o_ev = o_nv + align_up(sizeof(int32_t) * jobs, 256),
-         o_st = o_ev + align_up(sizeof(int32_t) * jobs, 256), o_left = o_st + align_up(jobs, 256),
-         o_best = o_left + align_up(jobs, 256), total = o_best + align_up(sizeof(int32_t) * batch, 256);
-  if ((rc = agt_scratch(ctx, 2, total, reinterpret_cast<void**>(&dr)))) return rc;
+  if ((rc = agt_scratch(ctx, SLOT_JOBS, jobs_bytes + align_up(sizeof(int32_t) * batch, 256), reinterpret_cast<void**>(&dr)))) return rc;
+  layout_jobs(&J, dr, jobs);
+  int32_t* d_best = reinterpret_cast<int32_t*>(dr + jobs_bytes);
   cudaStream_t st = ctx->stream, cp = ctx->copy_stream;
-  AGT_CUDA(ctx, cudaMemcpyAsync(dr + o_init, h_init, sizeof(double) * 6 * jobs, cudaMemcpyHostToDevice, st));
+  AGT_CUDA(ctx, cudaMemcpyAsync(J.init, h_init, sizeof(double) * 6 * jobs, cudaMemcpyHostToDevice, st));
   ctx->last_h2d_bytes += (int64_t)sizeof(double) * 6 * jobs;
   // the copy stream must not overwrite a buffer an earlier call on `st` may still read
   AGT_CUDA(ctx, cudaEventRecord(ctx->ev[3], st));
   AGT_CUDA(ctx, cudaStreamWaitEvent(cp, ctx->ev[3], 0));
   const int roi = ctx->roi_upload && !ctx->cam.has_dist;
-  ctx->host_frames_dev = nullptr;
+  refine_pass_desc d{roi ? PASS_ROI : PASS_WHOLE, h_frames, nullptr, h_init, w, h, levels, n_hyp, chunk,
+                     std::vector<agt_roi_rect>((size_t)batch)};
   if (roi) {
     cudaPointerAttributes attr;
     if (cudaPointerGetAttributes(&attr, h_frames) == cudaSuccess && attr.type == cudaMemoryTypeHost && attr.devicePointer)
-      ctx->host_frames_dev = static_cast<const uint8_t*>(attr.devicePointer);     // pinned + mapped: gather by kernel
+      d.frames_dev = static_cast<const uint8_t*>(attr.devicePointer);     // pinned + mapped: the gather kernel reads them
     else
-      cudaGetLastError();                                                          // pageable: per-frame 2-D copies
-    if (!ctx->host_frames_dev && ctx->upload_threads > 0 && (w & 15) == 0) {
-      // pageable frames: pinned staging (2 x one chunk of the largest rectangle a refinement can ask for) + packed device twin
-      agt_pyramid one;
-      layout_pyramid(&one, nullptr, w, h, levels, 1);
-      size_t need = 0, cur = 0;
-      for (int f = 0; f < batch; ++f) {
-        int X0, Y0, X1, Y1;
-        if (roi_rect_l0(ctx, one, h_init + (int64_t)f * n_hyp * 6, n_hyp, &X0, &Y0, &X1, &Y1)) cur += (size_t)(X1 - X0) * (Y1 - Y0);
-        if ((f + 1) % chunk == 0 || f + 1 == batch) { need = cur > need ? cur : need; cur = 0; }
-      }
-      need = align_up(need + 256, 4096);
-      if (ctx->stage_bytes < need) {
-        for (int k = 0; k < 2; ++k) { if (ctx->h_stage[k]) cudaFreeHost(ctx->h_stage[k]); ctx->h_stage[k] = nullptr; }
-        ctx->stage_bytes = 0;
-        for (int k = 0; k < 2; ++k) AGT_CUDA(ctx, cudaMallocHost(reinterpret_cast<void**>(&ctx->h_stage[k]), need));
-        ctx->stage_bytes = need;
-      }
-      void* dtmp;
-      if ((rc = agt_scratch(ctx, 6, 2 * ctx->stage_bytes, &dtmp))) return rc;
-      ctx->d_stage = static_cast<uint8_t*>(dtmp);
-      if (ctx->prect_capacity < batch) {
-        if (ctx->h_prects) cudaFreeHost(ctx->h_prects);
-        ctx->h_prects = nullptr; ctx->prect_capacity = 0;
-        AGT_CUDA(ctx, cudaMallocHost(reinterpret_cast<void**>(&ctx->h_prects), sizeof(agt_pack_rect) * (size_t)batch));
-        ctx->prect_capacity = batch;
-      }
-      if ((rc = agt_scratch(ctx, 4, sizeof(agt_pack_rect) * (size_t)batch, &dtmp))) return rc;
-      ctx->d_prects = static_cast<agt_pack_rect*>(dtmp);
-      for (int k = 0; k < 2; ++k)
-        if (!ctx->ev_stage[k]) AGT_CUDA(ctx, cudaEventCreateWithFlags(&ctx->ev_stage[k], cudaEventDisableTiming));
-    }
-    if (ctx->host_frames_dev) {
-      if (ctx->rect_capacity < batch) {
-        if (ctx->h_rects) cudaFreeHost(ctx->h_rects);
-        ctx->h_rects = nullptr; ctx->rect_capacity = 0;
-        AGT_CUDA(ctx, cudaMallocHost(reinterpret_cast<void**>(&ctx->h_rects), sizeof(agt_roi_rect) * (size_t)batch));
-        ctx->rect_capacity = batch;
-      }
-      void* dtmp;
-      if ((rc = agt_scratch(ctx, 4, sizeof(agt_roi_rect) * (size_t)batch, &dtmp))) return rc;
-      ctx->d_rects = static_cast<agt_roi_rect*>(dtmp);
-    }
+      cudaGetLastError();                                                  // pageable
+  } else {
+    for (int f = 0; f < batch; ++f) d.rects[(size_t)f] = {0, 0, w, h, f};
   }
-  if ((rc = refine_pass(ctx, h_frames, w, h, levels, nullptr, batch, n_hyp, roi, h_init, dr, o_init, o_pose, o_cost, o_nv, o_ev, o_st,
-                        o_left, chunk, buf)))
-    return rc;
+  if ((rc = refine_pass(ctx, d, J, buf))) return rc;
   if (trace) fprintf(stderr, "[agt] refine_host: first pass enqueued at %.3f ms (chunk %d, roi %d, gather %d)\n", since(), chunk, roi,
-                     ctx->host_frames_dev != nullptr);
+                     d.frames_dev != nullptr);
   if (roi) {
     // frames whose refinement read pixels outside the uploaded rectangle are redone from the whole frame,
     // so the result never depends on the ROI prediction
-    uint8_t* left = static_cast<uint8_t*>(malloc((size_t)jobs));
-    if (!left) AGT_FAIL(ctx, AGT_ERR_INVALID, "agt_refine_host: out of host memory");
-    cudaError_t e = cudaMemcpyAsync(left, dr + o_left, (size_t)jobs, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    if (e != cudaSuccess) { free(left); AGT_FAIL(ctx, AGT_ERR_CUDA, "agt_refine_host: %s", cudaGetErrorString(e)); }
-    int n_redo = 0;
-    int* ids = static_cast<int*>(malloc(sizeof(int) * (size_t)batch));
+    std::vector<uint8_t> left((size_t)jobs);
+    AGT_CUDA(ctx, cudaMemcpyAsync(left.data(), J.left, (size_t)jobs, cudaMemcpyDeviceToHost, st));
+    AGT_CUDA(ctx, cudaStreamSynchronize(st));
+    std::vector<int> ids;
     for (int f = 0; f < batch; ++f) {
       bool any = false;
-      for (int k = 0; k < n_hyp; ++k) any = any || left[(int64_t)f * n_hyp + k];
-      if (any) ids[n_redo++] = f;
+      for (int k = 0; k < n_hyp; ++k) any = any || left[(size_t)f * n_hyp + k];
+      if (any) ids.push_back(f);
     }
-    free(left);
-    ctx->last_redo_frames = n_redo;
+    const int n_redo = (int)ids.size();
     if (trace) fprintf(stderr, "[agt] refine_host: first pass done at %.3f ms, %d frames to redo\n", since(), n_redo);
     if (n_redo > 0) {
-      // compact the initial poses of the redo frames behind the main arrays and scatter the results back
+      // compact the initial poses of the redo frames into their own job arrays and scatter the results back
+      agt_jobs R;
+      const int64_t j2 = (int64_t)n_redo * n_hyp;
       uint8_t* dr2;
-      int64_t j2 = (int64_t)n_redo * n_hyp;
-      size_t p_init = 0, p_pose = p_init + align_up(sizeof(double) * 6 * j2, 256), p_cost = p_pose + align_up(sizeof(double) * 6 * j2, 256),
-             p_nv = p_cost + align_up(sizeof(float) * j2, 256), p_ev = p_nv + align_up(sizeof(int32_t) * j2, 256),
-             p_st = p_ev + align_up(sizeof(int32_t) * j2, 256), p_left = p_st + align_up(j2, 256), tot2 = p_left + align_up(j2, 256);
-      if ((rc = agt_scratch(ctx, 3, tot2, reinterpret_cast<void**>(&dr2)))) { free(ids); return rc; }
+      if ((rc = agt_scratch(ctx, SLOT_REDO_JOBS, layout_jobs(&R, nullptr, j2), reinterpret_cast<void**>(&dr2)))) return rc;
+      layout_jobs(&R, dr2, j2);
       for (int i = 0; i < n_redo; ++i)
-        cudaMemcpyAsync(dr2 + p_init + sizeof(double) * 6 * (size_t)i * n_hyp, h_init + (int64_t)ids[i] * n_hyp * 6,
-                        sizeof(double) * 6 * n_hyp, cudaMemcpyHostToDevice, st);
-      cudaEventRecord(ctx->ev[3], st);
-      cudaStreamWaitEvent(cp, ctx->ev[3], 0);
-      int chunk2 = chunk < n_redo ? chunk : n_redo;
-      rc = refine_pass(ctx, h_frames, w, h, levels, ids, n_redo, n_hyp, 0, h_init, dr2, p_init, p_pose, p_cost, p_nv, p_ev, p_st, p_left,
-                       chunk2, buf);
-      if (rc) { free(ids); return rc; }
+        AGT_CUDA(ctx, cudaMemcpyAsync(R.init + (int64_t)i * n_hyp * 6, h_init + (int64_t)ids[i] * n_hyp * 6, sizeof(double) * 6 * n_hyp,
+                                      cudaMemcpyHostToDevice, st));
+      AGT_CUDA(ctx, cudaEventRecord(ctx->ev[3], st));
+      AGT_CUDA(ctx, cudaStreamWaitEvent(cp, ctx->ev[3], 0));
+      d.kind = PASS_REDO;
+      d.chunk = chunk < n_redo ? chunk : n_redo;
+      d.rects.clear();
+      for (int f : ids) d.rects.push_back({0, 0, w, h, f});
+      if ((rc = refine_pass(ctx, d, R, buf))) return rc;
       for (int i = 0; i < n_redo; ++i) {
-        int64_t src = (int64_t)i * n_hyp, dst = (int64_t)ids[i] * n_hyp;
-        cudaMemcpyAsync(dr + o_pose + sizeof(double) * 6 * dst, dr2 + p_pose + sizeof(double) * 6 * src, sizeof(double) * 6 * n_hyp, cudaMemcpyDeviceToDevice, st);
-        cudaMemcpyAsync(dr + o_cost + sizeof(float) * dst, dr2 + p_cost + sizeof(float) * src, sizeof(float) * n_hyp, cudaMemcpyDeviceToDevice, st);
-        cudaMemcpyAsync(dr + o_nv + sizeof(int32_t) * dst, dr2 + p_nv + sizeof(int32_t) * src, sizeof(int32_t) * n_hyp, cudaMemcpyDeviceToDevice, st);
-        cudaMemcpyAsync(dr + o_ev + sizeof(int32_t) * dst, dr2 + p_ev + sizeof(int32_t) * src, sizeof(int32_t) * n_hyp, cudaMemcpyDeviceToDevice, st);
-        cudaMemcpyAsync(dr + o_st + dst, dr2 + p_st + src, (size_t)n_hyp, cudaMemcpyDeviceToDevice, st);
+        const int64_t from = (int64_t)i * n_hyp, to = (int64_t)ids[i] * n_hyp;
+        AGT_CUDA(ctx, cudaMemcpyAsync(J.pose + 6 * to, R.pose + 6 * from, sizeof(double) * 6 * n_hyp, cudaMemcpyDeviceToDevice, st));
+        AGT_CUDA(ctx, cudaMemcpyAsync(J.cost + to, R.cost + from, sizeof(float) * n_hyp, cudaMemcpyDeviceToDevice, st));
+        AGT_CUDA(ctx, cudaMemcpyAsync(J.n_valid + to, R.n_valid + from, sizeof(int32_t) * n_hyp, cudaMemcpyDeviceToDevice, st));
+        AGT_CUDA(ctx, cudaMemcpyAsync(J.evals + to, R.evals + from, sizeof(int32_t) * n_hyp, cudaMemcpyDeviceToDevice, st));
+        AGT_CUDA(ctx, cudaMemcpyAsync(J.status + to, R.status + from, (size_t)n_hyp, cudaMemcpyDeviceToDevice, st));
       }
     }
-    free(ids);
   }
   if (n_hyp > 1 && h_best) {
-    if ((rc = agt_select_best(ctx, reinterpret_cast<double*>(dr + o_pose), reinterpret_cast<float*>(dr + o_cost),
-                              reinterpret_cast<int32_t*>(dr + o_nv), n_hyp, reinterpret_cast<int32_t*>(dr + o_best), nullptr,
-                              batch)))
-      return rc;
-    AGT_CUDA(ctx, cudaMemcpyAsync(h_best, dr + o_best, sizeof(int32_t) * batch, cudaMemcpyDeviceToHost, st));
+    if ((rc = agt_select_best(ctx, J.pose, J.cost, J.n_valid, n_hyp, d_best, nullptr, batch))) return rc;
+    AGT_CUDA(ctx, cudaMemcpyAsync(h_best, d_best, sizeof(int32_t) * batch, cudaMemcpyDeviceToHost, st));
   }
-  AGT_CUDA(ctx, cudaMemcpyAsync(h_pose, dr + o_pose, sizeof(double) * 6 * jobs, cudaMemcpyDeviceToHost, st));
-  if (h_cost) AGT_CUDA(ctx, cudaMemcpyAsync(h_cost, dr + o_cost, sizeof(float) * jobs, cudaMemcpyDeviceToHost, st));
-  if (h_n_valid) AGT_CUDA(ctx, cudaMemcpyAsync(h_n_valid, dr + o_nv, sizeof(int32_t) * jobs, cudaMemcpyDeviceToHost, st));
-  if (h_evals) AGT_CUDA(ctx, cudaMemcpyAsync(h_evals, dr + o_ev, sizeof(int32_t) * jobs, cudaMemcpyDeviceToHost, st));
-  if (h_status) AGT_CUDA(ctx, cudaMemcpyAsync(h_status, dr + o_st, jobs, cudaMemcpyDeviceToHost, st));
+  AGT_CUDA(ctx, cudaMemcpyAsync(h_pose, J.pose, sizeof(double) * 6 * jobs, cudaMemcpyDeviceToHost, st));
+  if (h_cost) AGT_CUDA(ctx, cudaMemcpyAsync(h_cost, J.cost, sizeof(float) * jobs, cudaMemcpyDeviceToHost, st));
+  if (h_n_valid) AGT_CUDA(ctx, cudaMemcpyAsync(h_n_valid, J.n_valid, sizeof(int32_t) * jobs, cudaMemcpyDeviceToHost, st));
+  if (h_evals) AGT_CUDA(ctx, cudaMemcpyAsync(h_evals, J.evals, sizeof(int32_t) * jobs, cudaMemcpyDeviceToHost, st));
+  if (h_status) AGT_CUDA(ctx, cudaMemcpyAsync(h_status, J.status, jobs, cudaMemcpyDeviceToHost, st));
   AGT_CUDA(ctx, cudaStreamSynchronize(st));
   if (trace) fprintf(stderr, "[agt] refine_host: done at %.3f ms\n", since());
   return AGT_OK;
+} catch (const std::bad_alloc&) {            // the host lists of a call (ctx is set: nothing allocates before its check)
+  AGT_FAIL(ctx, AGT_ERR_INVALID, "agt_refine_host: out of host memory");
 }

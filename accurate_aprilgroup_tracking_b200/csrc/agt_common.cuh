@@ -50,20 +50,14 @@ struct agt_ctx {
   int lk_split_max;              // agt_lk of at most this many corners runs a warp per pyramid level (AGT_LK_SPLIT_MAX; 0: never)
   int roi_upload;                // agt_refine_host uploads only the rectangle a refinement can read
   int64_t last_h2d_bytes;        // host->device bytes of the last agt_refine_host call
-  int last_redo_frames;          // frames the last agt_refine_host call redid from the full frame
-  const uint8_t* host_frames_dev; // device alias of pinned host frames (NULL: pageable memory)
-  struct agt_roi_rect* h_rects;  // pinned ROI rectangle lists (double-buffered)
-  struct agt_roi_rect* d_rects;
-  int rect_capacity;
-  // pageable host frames: pinned staging (double-buffered) the upload threads pack ROI rows into, and its device twin
+  // pinned buffers of agt_refine_host (grow-only)
+  uint8_t* h_rects;              // rectangle list of the pass being uploaded: one agt_roi_rect or agt_pack_rect per frame
+  size_t rect_bytes;
+  // pageable host frames: pinned staging (double-buffered) the upload threads pack ROI rows into
   int upload_threads;            // 0: one 2-D copy per frame
   uint8_t* h_stage[2];
   size_t stage_bytes;
-  uint8_t* d_stage;
   cudaEvent_t ev_stage[2];
-  struct agt_pack_rect* h_prects;
-  struct agt_pack_rect* d_prects;
-  int prect_capacity;
   uint64_t* d_tag_codes;         // tag family (36-bit code words) of agt_decode_tags / agt_detect_tags
   int n_tag_codes;
   int tag_threshold;             // agt_set_tag_threshold: 0 auto, 1 one threshold per search window, 2 local white level
