@@ -101,6 +101,8 @@ PROTOTYPES = {
     "agt_set_upload_threads": (_I, [_VP, _I]),
     "agt_last_h2d_bytes": (_I64, [_VP]),
     "agt_refine_host": (_I, [_VP, _VP, _I, _I, _I, _I, _VP, _I, _VP, _VP, _VP, _VP, _VP, _VP]),
+    "agt_pose_covariance": (_I, [_VP, _PYR, _VP, _VP, _I, _VP, _VP, _VP, _VP, _VP, _VP, _I]),
+    "agt_pose_covariance_host": (_I, [_VP, _VP, _I, _I, _I, _I, _VP, _VP, _I, _VP, _VP, _VP, _VP, _VP]),
 }
 
 

@@ -10,6 +10,9 @@ reference names but does not yet contain can be switched on:
                         used when fewer than two tags are detected (SURVEY.md 3.4 / 9.2)
   ``use_dense_refine``  dense photometric refinement of every accepted pose before it becomes
                         ``prev_transform`` (SURVEY.md 9.4)
+  ``pose_covariance``   with ``use_dense_refine``: after each frame ``self.pose_covariance`` holds the 6x6
+                        covariance of the refined pose (rotation in radians first, then translation in
+                        metres; ``HostContext.pose_covariance``), or None when the frame was not refined
 
 Both default to False, which reproduces the reference's behaviour frame by frame,
 including the in-place write of solvePnP into the guess arrays and the resulting
@@ -60,7 +63,7 @@ class PoseDetector(TransformHelper, Draw):
     JSON_FILE = 'april_group.json'
 
     def __init__(self, logger, mtx, dist, enhance_ape, use_lk: bool = False, use_dense_refine: bool = False,
-                 surface_model=None, device: int = 0):
+                 surface_model=None, device: int = 0, pose_covariance: bool = False):
         TransformHelper.__init__(self, logger, mtx, dist)
         Draw.__init__(self, logger)
         self.logger = logger
@@ -75,6 +78,10 @@ class PoseDetector(TransformHelper, Draw):
         self.enhance_ape = enhance_ape
         self.use_lk = use_lk
         self.use_dense_refine = use_dense_refine
+        if pose_covariance and not use_dense_refine:
+            raise ValueError("pose_covariance needs use_dense_refine: it is the covariance of the refined pose")
+        self.want_pose_covariance = pose_covariance
+        self.pose_covariance = None    # 6x6 covariance of the last frame's refined pose (want_pose_covariance)
         self._agt = agt_cv.default_context() if device == 0 else agt_cv.HostContext(device)   # raises without a B200
         self._gray = None
         self._prev_gray = None
@@ -258,6 +265,10 @@ class PoseDetector(TransformHelper, Draw):
                              "first, as the reference's capture loop does (detect_pose.py:678)")
         ok, rvec, tvec, _, _ = self._agt.refine_pose(self._gray, transformation[0], transformation[1], self._gray_mtx)
         if ok:
+            if self.want_pose_covariance:
+                init = np.concatenate([np.asarray(v, dtype=np.float64).reshape(3) for v in transformation])
+                pose = np.concatenate([rvec.reshape(3), tvec.reshape(3)])
+                self.pose_covariance = self._agt.pose_covariance(self._gray, init, pose, self._gray_mtx)["cov"][0, 0]
             transformation[0].reshape(-1)[:] = rvec.reshape(-1)
             transformation[1].reshape(-1)[:] = tvec.reshape(-1)
 
@@ -279,6 +290,7 @@ class PoseDetector(TransformHelper, Draw):
 
     def _detect_and_get_pose(self, frame: np.ndarray) -> None:
         self.img = frame
+        self.pose_covariance = None
         height, width = frame.shape[:2]
         self.draw_frame = np.zeros(shape=[height, width, 3], dtype=np.uint8)
         gray = self._set_gray(frame)

@@ -33,9 +33,13 @@ class BatchedPoseDetector:
 
     def __init__(self, ctx: AgtContext, n_streams: int, width: int, height: int, obj_pts: np.ndarray,
                  enhance_ape: bool = True, use_lk: bool = True, use_dense_refine: bool = True, levels: int = 4,
-                 use_graphs: bool = True, tag_ids=None):
+                 use_graphs: bool = True, tag_ids=None, pose_covariance: bool = False):
         """``obj_pts`` [4T,3]: the group's corners in JSON key order (``PoseDetector.all_objpts``); ``tag_ids``: the ids in the
-        same order (``list(PoseDetector.extrinsics)``), default 0..T-1 - ``pack`` puts detections where their object points are."""
+        same order (``list(PoseDetector.extrinsics)``), default 0..T-1 - ``pack`` puts detections where their object points are.
+        ``pose_covariance`` (with ``use_dense_refine``): one more launch per step after K4, masked by the same gate, puts the
+        covariance of every refined pose (agt_pose_covariance) into the step's ``covariance`` [S,6,6] and ``covariance_ok`` [S]
+        (0 where the frame was not refined or the covariance is undefined; ``covariance`` is not written for frames that were
+        not refined)."""
         t = ctx.torch
         if obj_pts.shape[0] % 4:
             raise ValueError("obj_pts must hold four corners per tag")
@@ -44,6 +48,9 @@ class BatchedPoseDetector:
             raise ValueError(f"{len(self.tag_pos)} tag ids for {obj_pts.shape[0] // 4} tags of object points")
         self.ctx, self.n, self.enhance_ape = ctx, int(n_streams), enhance_ape
         self.use_lk, self.use_dense_refine = use_lk, use_dense_refine
+        if pose_covariance and not use_dense_refine:
+            raise ValueError("pose_covariance needs use_dense_refine: it is the covariance of the refined pose")
+        self.pose_covariance = bool(pose_covariance)
         self.n_pts = int(obj_pts.shape[0])
         self.obj = ctx._dev(obj_pts, t.float32)
         # three frame slots: a step reads the current and the previous one, the third is free to receive the next frame while
@@ -173,11 +180,19 @@ class BatchedPoseDetector:
                                 ("left_roi", t.uint8))}
             out["status"] = fr["status"]                                          # masked frames keep status 0: pose unused
             refined = ctx.refine(cur, pose.reshape(self.n, 1, 6), 1, mask=fr["gate"], out=out)   # K4
+        cov = None
+        if self.pose_covariance:
+            cov = {"cov": t.empty((self.n, 1, 6, 6), dtype=t.float64, device=ctx.tdev),
+                   "ok": t.zeros((self.n, 1), dtype=t.uint8, device=ctx.tdev)}
+            ctx.pose_covariance(cur, pose.reshape(self.n, 1, 6), refined["pose"], 1, mask=fr["gate"], out=cov)
         # K0 with the refined pose where there is one; the corners of the accepted frame feed the next LK step
         accepted, flag, pose_out = ctx.ape_commit(self.state, ntg, pose, ok, err, refined, img, val, self.prev_pts,
                                                   self.prev_valid, self.enhance_ape)
-        return {"pose": pose_out, "accepted": accepted, "error_flag": flag, "reproj_err": err,
-                "n_tags": ntg, "tracked_tags": tracked_tags, "refine": refined}
+        res = {"pose": pose_out, "accepted": accepted, "error_flag": flag, "reproj_err": err,
+               "n_tags": ntg, "tracked_tags": tracked_tags, "refine": refined}
+        if cov is not None:
+            res["covariance"], res["covariance_ok"] = cov["cov"].reshape(self.n, 6, 6), cov["ok"].reshape(self.n)
+        return res
 
     def step_frames(self, frames=None, min_margin: float = 50.0, refine_win: int = 4, max_tags: int = 32, check_ids: bool = False,
                     track_window: bool = True, track_margin: int = 48):

@@ -512,6 +512,35 @@ class AgtContext:
                        self._p(out["left_roi"]), b))
         return out
 
+    def pose_covariance(self, pyr: Pyramid, init, pose, n_hyp: int = 1, mask=None, out=None):
+        """Covariance of refined poses (agt_pose_covariance): the refinement's cost function, fixed by ``init`` [B,H,6] as
+        ``refine`` fixes it, evaluated once at ``pose`` [B,H,6] (normally the refined pose) -> dict(cov [B,H,6,6] f64 =
+        s^2 H^-1, info [B,H,6,6] f64 = H = J^T J, sigma2 [B,H] f32 = s^2 = 2c / (n_valid - 6), n_valid [B,H] i32, ok [B,H] u8).
+        Tangent order: rotation (left perturbation R <- exp(w) R, radians), then translation (metres).  ok = 0 (cov NaN)
+        when n_valid <= 6 or H is not positive definite.  mask [B] u8 / ``out`` as for ``refine``: frames with mask 0 are
+        skipped and their outputs left as they are."""
+        t = self.torch
+        if n_hyp < 1:
+            raise ValueError(f"pose_covariance: n_hyp must be at least 1 (got {n_hyp})")
+        ini = self._dev(init, t.float64).reshape(-1, n_hyp, 6)
+        b = int(ini.shape[0])
+        if b > pyr.batch:
+            raise ValueError(f"pose_covariance: {b} frames of poses for a pyramid of {pyr.batch}")
+        ps = self._dev(pose, t.float64).reshape(b, n_hyp, 6)
+        if out is None:
+            fresh = t.zeros if mask is not None else t.empty
+            out = {"cov": fresh((b, n_hyp, 6, 6), dtype=t.float64, device=self.tdev),
+                   "info": fresh((b, n_hyp, 6, 6), dtype=t.float64, device=self.tdev),
+                   "sigma2": fresh((b, n_hyp), dtype=t.float32, device=self.tdev),
+                   "n_valid": fresh((b, n_hyp), dtype=t.int32, device=self.tdev),
+                   "ok": fresh((b, n_hyp), dtype=t.uint8, device=self.tdev)}
+        msk = self._dev(mask, t.uint8) if mask is not None else None
+        self._use_current_stream()
+        self._check(self.lib.agt_pose_covariance(self.h, C.byref(pyr.desc), self._p(ini), self._p(ps), n_hyp, self._p(msk),
+                                                 self._p(out["cov"]), self._p(out.get("info")), self._p(out.get("sigma2")),
+                                                 self._p(out.get("n_valid")), self._p(out["ok"]), b))
+        return out
+
     def dpr_rects(self, pyr: Pyramid, init, n_hyp: int = 1, batch: Optional[int] = None):
         """Level-0 rectangle [B,4] i32 (x0,y0,x1,y1) each frame's refinements can read."""
         t = self.torch

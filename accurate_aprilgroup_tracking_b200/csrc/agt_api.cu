@@ -732,3 +732,44 @@ extern "C" int agt_refine_host(agt_ctx* ctx, const uint8_t* h_frames, int w, int
 } catch (const std::bad_alloc&) {            // the host lists of a call (ctx is set: nothing allocates before its check)
   AGT_FAIL(ctx, AGT_ERR_INVALID, "agt_refine_host: out of host memory");
 }
+
+extern "C" int agt_pose_covariance_host(agt_ctx* ctx, const uint8_t* h_frames, int w, int h, int levels, int batch, const double* h_init,
+                                        const double* h_pose, int n_hyp, double* h_cov, double* h_info, float* h_sigma2,
+                                        int32_t* h_n_valid, uint8_t* h_ok) {
+  if (!ctx) return AGT_ERR_INVALID;
+  if (!h_frames || !h_init || !h_pose || !h_cov || !h_ok || w < 1 || h < 1 || levels < 1 || levels > AGT_MAX_LEVELS || batch < 0 ||
+      n_hyp < 1)
+    AGT_FAIL(ctx, AGT_ERR_INVALID, "agt_pose_covariance_host: bad arguments");
+  if (batch == 0) return AGT_OK;
+  AGT_CUDA(ctx, cudaSetDevice(ctx->device));
+  // whole frames, one pyramid for the batch (SLOT_CHUNK0), then the poses and the outputs (SLOT_JOBS)
+  agt_pyramid p;
+  const int64_t pyr_bytes = layout_pyramid(&p, nullptr, w, h, levels, batch);
+  const int64_t jobs = (int64_t)batch * n_hyp;
+  const int64_t o_pose = align_up(sizeof(double) * 6 * jobs, 256), o_cov = o_pose + o_pose, o_info = o_cov + align_up(sizeof(double) * 36 * jobs, 256),
+                o_s2 = o_info + align_up(sizeof(double) * 36 * jobs, 256), o_nv = o_s2 + align_up(sizeof(float) * jobs, 256),
+                o_ok = o_nv + align_up(sizeof(int32_t) * jobs, 256), total = o_ok + align_up(jobs, 256);
+  uint8_t *dp, *d;
+  int rc;
+  if ((rc = agt_scratch(ctx, SLOT_CHUNK0, (size_t)pyr_bytes, reinterpret_cast<void**>(&dp)))) return rc;
+  if ((rc = agt_scratch(ctx, SLOT_JOBS, (size_t)total, reinterpret_cast<void**>(&d)))) return rc;
+  layout_pyramid(&p, dp, w, h, levels, batch);
+  cudaStream_t st = ctx->stream;
+  // level 0 rows of consecutive frames are consecutive (frame_stride = pitch * h): one 2-D copy for the batch
+  AGT_CUDA(ctx, cudaMemcpy2DAsync(p.data[0], (size_t)p.pitch[0], h_frames, (size_t)w, (size_t)w, (size_t)h * batch,
+                                  cudaMemcpyHostToDevice, st));
+  AGT_CUDA(ctx, cudaMemcpyAsync(d, h_init, sizeof(double) * 6 * jobs, cudaMemcpyHostToDevice, st));
+  AGT_CUDA(ctx, cudaMemcpyAsync(d + o_pose, h_pose, sizeof(double) * 6 * jobs, cudaMemcpyHostToDevice, st));
+  if ((rc = agt_build_pyramid(ctx, &p, batch))) return rc;
+  if ((rc = agt_pose_covariance(ctx, &p, reinterpret_cast<const double*>(d), reinterpret_cast<const double*>(d + o_pose), n_hyp, nullptr,
+                                reinterpret_cast<double*>(d + o_cov), reinterpret_cast<double*>(d + o_info),
+                                reinterpret_cast<float*>(d + o_s2), reinterpret_cast<int32_t*>(d + o_nv), d + o_ok, batch)))
+    return rc;
+  AGT_CUDA(ctx, cudaMemcpyAsync(h_cov, d + o_cov, sizeof(double) * 36 * jobs, cudaMemcpyDeviceToHost, st));
+  if (h_info) AGT_CUDA(ctx, cudaMemcpyAsync(h_info, d + o_info, sizeof(double) * 36 * jobs, cudaMemcpyDeviceToHost, st));
+  if (h_sigma2) AGT_CUDA(ctx, cudaMemcpyAsync(h_sigma2, d + o_s2, sizeof(float) * jobs, cudaMemcpyDeviceToHost, st));
+  if (h_n_valid) AGT_CUDA(ctx, cudaMemcpyAsync(h_n_valid, d + o_nv, sizeof(int32_t) * jobs, cudaMemcpyDeviceToHost, st));
+  AGT_CUDA(ctx, cudaMemcpyAsync(h_ok, d + o_ok, (size_t)jobs, cudaMemcpyDeviceToHost, st));
+  AGT_CUDA(ctx, cudaStreamSynchronize(st));
+  return AGT_OK;
+}

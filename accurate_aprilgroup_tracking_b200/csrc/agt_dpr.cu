@@ -959,6 +959,202 @@ __global__ void select_best_kernel(const double* __restrict__ pose, const float*
   if (best_pose && lane < 6) best_pose[(int64_t)f * 6 + lane] = pose[((int64_t)f * n_hyp + bi) * 6 + lane];
 }
 
+// ---- covariance of a finished refinement (agt_pose_covariance) ----------------------------------------------------
+// One evaluation of the refinement's cost function at a given pose: the level and the active tags are fixed by the
+// initial pose exactly as in dpr_kernel (dpr_prep_warp), the samples are projected, the 4x4 footprint is fetched from
+// the level image and the Scharr taps come from the same dp4a coefficient words.  No shared-memory tile: a single pass
+// reads each footprint once, mostly from L1.  It reads exactly the pixels the refinement's last evaluation read, so it is
+// valid on a full pyramid, and on a region-of-interest or fused pyramid for every refinement that reported left_roi = 0.  The projection and everything after the bilinear interpolation run in
+// float64 and so do the sums, which keeps the inverse clear of float32 rounding; the intensity and gradient
+// interpolation stay in float32 like the refinement's.  A CTA per (frame, hypothesis), each thread a strided share of
+// the active samples in sequence order, a fixed reduction tree: the result does not depend on the batch or its position.
+constexpr int COV_THREADS = 128;                 // (CTAs of 256 and a warp per pose: not measured; profiles/r03_pose_cov.log)
+constexpr int COV_WARPS = COV_THREADS / 32;
+constexpr int COV_NSUM = 23;                     // 21 H (packed upper triangle by rows) + cost + count
+
+// Cholesky of the SPD 6x6 matrix H (packed upper triangle) and H^-1 (full, row-major) from it.  False if H is not
+// positive definite.
+__device__ bool cov_spd_inverse(const double* h, double inv[36]) {
+  double L[6][6];
+  for (int j = 0; j < 6; ++j) {
+    double d = h[agt_hk(j, j)];
+    for (int k = 0; k < j; ++k) d -= L[j][k] * L[j][k];
+    if (!(d > 0.0) || !isfinite(d)) return false;
+    L[j][j] = sqrt(d);
+    for (int i = j + 1; i < 6; ++i) {
+      double v = h[agt_hk(j, i)];
+      for (int k = 0; k < j; ++k) v -= L[i][k] * L[j][k];
+      L[i][j] = v / L[j][j];
+    }
+  }
+  // M = L^-1 (lower triangular), then H^-1 = M^T M
+  double M[6][6];
+  for (int c = 0; c < 6; ++c)
+    for (int r = 0; r < 6; ++r) {
+      if (r < c) { M[r][c] = 0.0; continue; }
+      double v = r == c ? 1.0 : 0.0;
+      for (int k = c; k < r; ++k) v -= L[r][k] * M[k][c];
+      M[r][c] = v / L[r][r];
+    }
+  for (int i = 0; i < 6; ++i)
+    for (int j = i; j < 6; ++j) {
+      double v = 0.0;
+      for (int k = j; k < 6; ++k) v += M[k][i] * M[k][j];
+      inv[i * 6 + j] = v; inv[j * 6 + i] = v;
+    }
+  return true;
+}
+
+__global__ void __launch_bounds__(COV_THREADS)
+pose_cov_kernel(agt_pyramid pyr, agt_camera cam, const float4* __restrict__ samples, agt_model model, const double* __restrict__ init,
+                const double* __restrict__ pose, int n_hyp, const uint8_t* __restrict__ mask, double* __restrict__ cov_out,
+                double* __restrict__ info_out, float* __restrict__ sigma2_out, int32_t* __restrict__ nvalid_out,
+                uint8_t* __restrict__ ok_out) {
+  __shared__ DprJob job_s;
+  __shared__ double Pd[12];                      // evaluation pose: rotation (row-major) + translation
+  __shared__ int act_begin[AGT_MAX_TAGS], act_prefix[AGT_MAX_TAGS + 1];
+  __shared__ double wsum[COV_WARPS][COV_NSUM];
+  const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+  const int64_t job = blockIdx.x;
+  if (mask != nullptr && mask[job / n_hyp] == 0) return;      // skipped frame: none of its outputs is written
+  const int64_t frame = job / n_hyp;
+  if (wid == 0) dpr_prep_warp(pyr, cam, model, init + job * 6, &job_s, lane);
+  if (wid == 1 && lane == 0) {
+    const double* p = pose + job * 6;
+    const double r[3] = {p[0], p[1], p[2]};
+    agt_rodrigues(r, Pd);
+    Pd[9] = p[3]; Pd[10] = p[4]; Pd[11] = p[5];
+  }
+  __syncthreads();
+  if (tid == 0) {                                // active tags (visibility frozen at the initial pose)
+    int na = 0, pre = 0;
+    for (int k = 0; k < model.n_tags; ++k) {
+      if (job_s.active >> k & 1u) {
+        act_begin[na] = model.tag_begin[k];
+        act_prefix[na] = pre;
+        pre += model.tag_begin[k + 1] - model.tag_begin[k];
+        ++na;
+      }
+    }
+    for (int k = na; k <= AGT_MAX_TAGS; ++k) act_prefix[k] = pre;
+  }
+  __syncthreads();
+  const int lvl = job_s.level;
+  const int lw = pyr.width[lvl], lh = pyr.height[lvl];
+  const int64_t lpitch = pyr.pitch[lvl];
+  const uint8_t* limg = pyr.data[lvl] + frame * pyr.frame_stride[lvl];
+  // aligned 32-bit row words need a 4-byte aligned level; the word right of the footprint must lie inside the row
+  const bool words = ((lpitch & 3) == 0) && ((reinterpret_cast<uintptr_t>(limg) & 3) == 0);
+  const double sc = 1.0 / (double)(1 << lvl);
+  const double fxl = cam.fx * sc, fyl = cam.fy * sc, cxl = cam.cx * sc, cyl = cam.cy * sc;
+  const double gsc = sc / 32.0;
+  double R[9], t[3];
+#pragma unroll
+  for (int i = 0; i < 9; ++i) R[i] = Pd[i];
+  t[0] = Pd[9]; t[1] = Pd[10]; t[2] = Pd[11];
+  const int cDX0_3 = kCoef[0], cDX0_10 = kCoef[1], cDX1_3 = kCoef[2], cDX1_10 = kCoef[3], cSM0 = kCoef[4], cSM1 = kCoef[5],
+            cSM0_NEG = kCoef[6], cSM1_NEG = kCoef[7];
+
+  double hs[21];
+#pragma unroll
+  for (int k = 0; k < 21; ++k) hs[k] = 0.0;
+  double cost = 0.0;
+  int cnt = 0;
+  const int n_act = act_prefix[AGT_MAX_TAGS];
+  int seg = 0;
+  for (int j = tid; j < n_act; j += COV_THREADS) {
+    while (j >= act_prefix[seg + 1]) ++seg;
+    const float4 sm = __ldg(&samples[act_begin[seg] + (j - act_prefix[seg])]);
+    const double sx = sm.x, sy = sm.y, sz = sm.z;
+    const double Yx = fma(R[0], sx, fma(R[1], sy, R[2] * sz));
+    const double Yy = fma(R[3], sx, fma(R[4], sy, R[5] * sz));
+    const double Yz = fma(R[6], sx, fma(R[7], sy, R[8] * sz));
+    const double X = Yx + t[0], Y = Yy + t[1], Z = Yz + t[2];
+    if (!(Z > 1e-6)) continue;
+    const double iz = 1.0 / Z;
+    const double ul = fma(fxl * X, iz, cxl), vl = fma(fyl * Y, iz, cyl);
+    const double fu = floor(ul), fv = floor(vl);
+    // valid <=> 1 <= floor(ul) <= lw-3 and 1 <= floor(vl) <= lh-3 (compared in float64: no integer overflow far away)
+    if (!(fu >= 1.0 && fu <= (double)(lw - 3) && fv >= 1.0 && fv <= (double)(lh - 3))) continue;
+    const int x0 = (int)fu, y0 = (int)fv;
+    const uint8_t* g = limg + (int64_t)(y0 - 1) * lpitch + (x0 - 1);
+    uint32_t row[4];
+    const int a0 = (x0 - 1) & ~3;
+    if (words && a0 + 8 <= lpitch) {
+      const uint32_t* wp = reinterpret_cast<const uint32_t*>(limg + (int64_t)(y0 - 1) * lpitch + a0);
+      const uint32_t sel = 0x3210 + 0x1111 * ((x0 - 1) & 3);
+      const int64_t wstep = lpitch >> 2;
+#pragma unroll
+      for (int r = 0; r < 4; ++r) row[r] = __byte_perm(__ldg(wp + r * wstep), __ldg(wp + r * wstep + 1), sel);
+    } else {
+#pragma unroll
+      for (int r = 0; r < 4; ++r)
+        row[r] = (uint32_t)__ldg(g + r * lpitch) | ((uint32_t)__ldg(g + r * lpitch + 1) << 8) |
+                 ((uint32_t)__ldg(g + r * lpitch + 2) << 16) | ((uint32_t)__ldg(g + r * lpitch + 3) << 24);
+    }
+    // Scharr (dx, dy) at (x0,y0) (x0+1,y0) (x0,y0+1) (x0+1,y0+1): integers, as cv::Scharr
+    const int gx00 = dp4c(row[2], cDX0_3, dp4c(row[1], cDX0_10, dp4c(row[0], cDX0_3, 0)));
+    const int gy00 = dp4c(row[2], cSM0, dp4c(row[0], cSM0_NEG, 0));
+    const int gx01 = dp4c(row[2], cDX1_3, dp4c(row[1], cDX1_10, dp4c(row[0], cDX1_3, 0)));
+    const int gy01 = dp4c(row[2], cSM1, dp4c(row[0], cSM1_NEG, 0));
+    const int gx10 = dp4c(row[3], cDX0_3, dp4c(row[2], cDX0_10, dp4c(row[1], cDX0_3, 0)));
+    const int gy10 = dp4c(row[3], cSM0, dp4c(row[1], cSM0_NEG, 0));
+    const int gx11 = dp4c(row[3], cDX1_3, dp4c(row[2], cDX1_10, dp4c(row[1], cDX1_3, 0)));
+    const int gy11 = dp4c(row[3], cSM1, dp4c(row[1], cSM1_NEG, 0));
+    const float a = (float)(ul - fu), b = (float)(vl - fv);
+    const float w00 = (1.f - a) * (1.f - b), w01 = a * (1.f - b), w10 = (1.f - a) * b, w11 = a * b;
+    const float i00 = (float)((row[1] >> 8) & 0xffu), i01 = (float)((row[1] >> 16) & 0xffu);
+    const float i10 = (float)((row[2] >> 8) & 0xffu), i11 = (float)((row[2] >> 16) & 0xffu);
+    const float I = fmaf(w11, i11, fmaf(w10, i10, fmaf(w01, i01, w00 * i00)));
+    const float Gx = fmaf(w11, (float)gx11, fmaf(w10, (float)gx10, fmaf(w01, (float)gx01, w00 * (float)gx00)));
+    const float Gy = fmaf(w11, (float)gy11, fmaf(w10, (float)gy10, fmaf(w01, (float)gy01, w00 * (float)gy00)));
+    const double r = (double)I - (double)sm.w;
+    const double g0 = (double)Gx * gsc * cam.fx * iz, g1 = (double)Gy * gsc * cam.fy * iz;
+    const double g2 = -(g0 * X + g1 * Y) * iz;
+    const double J[6] = {Yy * g2 - Yz * g1, Yz * g0 - Yx * g2, Yx * g1 - Yy * g0, g0, g1, g2};
+#pragma unroll
+    for (int p = 0; p < 6; ++p)
+#pragma unroll
+      for (int q = p; q < 6; ++q) hs[agt_hk(p, q)] = fma(J[p], J[q], hs[agt_hk(p, q)]);
+    cost = fma(r, r, cost);
+    ++cnt;
+  }
+  // fixed reduction tree: butterfly within the warp, warps in order
+#pragma unroll
+  for (int k = 0; k < 21; ++k) hs[k] = agt_warp_sum(hs[k]);
+  cost = agt_warp_sum(cost);
+  cnt = __reduce_add_sync(0xffffffffu, cnt);
+  if (lane == 0) {
+#pragma unroll
+    for (int k = 0; k < 21; ++k) wsum[wid][k] = hs[k];
+    wsum[wid][21] = cost;
+    wsum[wid][22] = (double)cnt;
+  }
+  __syncthreads();
+  if (tid != 0) return;
+  double tot[COV_NSUM];
+  for (int k = 0; k < COV_NSUM; ++k) {
+    double v = 0.0;
+    for (int w = 0; w < COV_WARPS; ++w) v += wsum[w][k];
+    tot[k] = v;
+  }
+  const int n = (int)tot[22];
+  const double c = 0.5 * tot[21];
+  const double s2 = n > 6 ? 2.0 * c / (double)(n - 6) : nan("");
+  double inv[36];
+  const bool ok = n > 6 && cov_spd_inverse(tot, inv);
+  double* co = cov_out + job * 36;
+  for (int k = 0; k < 36; ++k) co[k] = ok ? s2 * inv[k] : nan("");
+  if (info_out) {
+    double* io = info_out + job * 36;
+    for (int p = 0; p < 6; ++p)
+      for (int q = 0; q < 6; ++q) io[p * 6 + q] = tot[p <= q ? agt_hk(p, q) : agt_hk(q, p)];
+  }
+  if (sigma2_out) sigma2_out[job] = (float)s2;
+  if (nvalid_out) nvalid_out[job] = n;
+  ok_out[job] = ok ? 1 : 0;
+}
+
 }  // namespace
 
 static int refine_impl(agt_ctx* ctx, const agt_pyramid* pyr, const double* d_init, int n_hyp, const uint8_t* d_mask,
@@ -1038,6 +1234,24 @@ extern "C" int agt_refine_fused(agt_ctx* ctx, const agt_pyramid* pyr, const doub
                                 double* d_pose, float* d_cost, int32_t* d_n_valid, int32_t* d_evals, uint8_t* d_status,
                                 uint8_t* d_left_roi, int batch) {
   return refine_impl(ctx, pyr, d_init, n_hyp, d_mask, d_pose, d_cost, d_n_valid, d_evals, d_status, d_left_roi, batch, 1);
+}
+
+extern "C" int agt_pose_covariance(agt_ctx* ctx, const agt_pyramid* pyr, const double* d_init, const double* d_pose, int n_hyp,
+                                   const uint8_t* d_mask, double* d_cov, double* d_info, float* d_sigma2, int32_t* d_n_valid,
+                                   uint8_t* d_ok, int batch) {
+  if (!ctx) return AGT_ERR_INVALID;
+  if (!pyr || !d_init || !d_pose || !d_cov || !d_ok || n_hyp < 1 || batch < 0)
+    AGT_FAIL(ctx, AGT_ERR_INVALID, "agt_pose_covariance: bad arguments");
+  if (batch == 0) return AGT_OK;
+  if (!ctx->camera_set || !ctx->model_set) AGT_FAIL(ctx, AGT_ERR_NOT_READY, "agt_pose_covariance: camera and surface model must be set");
+  if (pyr->levels < 1 || pyr->levels > AGT_MAX_LEVELS) AGT_FAIL(ctx, AGT_ERR_INVALID, "agt_pose_covariance: bad pyramid descriptor");
+  if (ctx->cam.has_dist) AGT_FAIL(ctx, AGT_ERR_INVALID, "agt_pose_covariance: lens distortion is not supported; undistort the frame first");
+  const int64_t jobs = (int64_t)batch * n_hyp;
+  if (jobs > 0x7fffffffLL) AGT_FAIL(ctx, AGT_ERR_INVALID, "agt_pose_covariance: batch*n_hyp too large");
+  pose_cov_kernel<<<(unsigned)jobs, COV_THREADS, 0, ctx->stream>>>(*pyr, ctx->cam, ctx->model.samples, ctx->model, d_init, d_pose, n_hyp,
+                                                                  d_mask, d_cov, d_info, d_sigma2, d_n_valid, d_ok);
+  AGT_LAUNCH_CHECK(ctx);
+  return AGT_OK;
 }
 
 extern "C" int agt_select_best(agt_ctx* ctx, const double* d_pose, const float* d_cost, const int32_t* d_n_valid,

@@ -321,6 +321,29 @@ class HostContext:
                                              best.ctypes.data if best is not None else None))
         return {"pose": pose, "cost": cost, "n_valid": nv, "evals": ev, "status": st, "best": best}
 
+    def pose_covariance(self, frames, init, pose, cameraMatrix, n_hyp: int = 1, levels: int = 4):
+        """Covariance of refined poses (agt_pose_covariance_host): frames [B,H,W] u8 (host, whole frames are uploaded), init /
+        pose [B,n_hyp,6] f64 - the refinement's start, which fixes its cost function, and the pose to evaluate at.
+        -> dict(cov [B,n_hyp,6,6] = s^2 H^-1, info [B,n_hyp,6,6] = H, sigma2 [B,n_hyp] f32, n_valid [B,n_hyp] i32, ok [B,n_hyp] bool);
+        rotation (radians) before translation (metres); cov is NaN where ok is False."""
+        if not self._model_set:
+            raise RuntimeError("set_model() must be called before pose_covariance()")
+        self.use_camera(cameraMatrix, None)
+        fr = np.ascontiguousarray(frames, dtype=np.uint8)
+        if fr.ndim == 2:
+            fr = fr[None]
+        b, h, w = fr.shape
+        ini = np.ascontiguousarray(np.asarray(init, dtype=np.float64).reshape(b, n_hyp, 6))
+        ps = np.ascontiguousarray(np.asarray(pose, dtype=np.float64).reshape(b, n_hyp, 6))
+        cov = np.zeros((b, n_hyp, 6, 6), np.float64)
+        info = np.zeros((b, n_hyp, 6, 6), np.float64)
+        s2 = np.zeros((b, n_hyp), np.float32)
+        nv = np.zeros((b, n_hyp), np.int32)
+        ok = np.zeros((b, n_hyp), np.uint8)
+        self._check(self.lib.agt_pose_covariance_host(self.h, fr.ctypes.data, w, h, levels, b, ini.ctypes.data, ps.ctypes.data, n_hyp,
+                                                      cov.ctypes.data, info.ctypes.data, s2.ctypes.data, nv.ctypes.data, ok.ctypes.data))
+        return {"cov": cov, "info": info, "sigma2": s2, "n_valid": nv, "ok": ok.astype(bool)}
+
     def refine_pose(self, gray, rvec, tvec, cameraMatrix):
         """Single frame: -> (ok, rvec (3,1), tvec (3,1), cost, evals)."""
         init = np.concatenate([np.asarray(rvec, dtype=np.float64).reshape(3), np.asarray(tvec, dtype=np.float64).reshape(3)])

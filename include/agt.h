@@ -319,6 +319,25 @@ int agt_refine_fused(agt_ctx* ctx, const agt_pyramid* pyr, const double* d_init,
 int agt_dpr_rects(agt_ctx* ctx, const agt_pyramid* pyr, const double* d_init, int n_hyp, int32_t* d_rects, int batch);
 /* d_out[b] = any(d_flags[b*stride .. b*stride+stride-1]) */
 int agt_any_flag(agt_ctx* ctx, const uint8_t* d_flags, int stride, uint8_t* d_out, int batch);
+/* Covariance of a refined pose: one evaluation of the refinement's cost function at d_pose[batch][n_hyp][6], the
+ * cost function being the one agt_refine fixes from d_init[batch][n_hyp][6] (pyramid level and visible tags decided
+ * at the initial pose).  With J the n_valid x 6 Jacobian of the residuals in the refinement's tangent convention -
+ * left perturbation R <- exp(w) R, then t <- t + dt; rotation block first (radians), then translation (metres) -
+ * and c = 1/2 sum r^2:
+ *   d_info[b][h][36] = H = J^T J (row-major, may be NULL),
+ *   d_sigma2[b][h]   = s^2 = 2c / (n_valid - 6) (float32, may be NULL; NaN when n_valid <= 6),
+ *   d_n_valid[b][h]  = samples in the evaluation (may be NULL),
+ *   d_cov[b][h][36]  = Sigma = s^2 H^-1 (row-major, float64),
+ *   d_ok[b][h]       = 1, or 0 when n_valid <= 6 or H is not positive definite; Sigma is then NaN.
+ * Sigma is the Gauss-Newton covariance of the estimate under independent residuals of equal variance; it is not a
+ * bound on the error against the true pose (the estimator's bias is not in it; DESIGN.md section 2).
+ * d_mask[batch] (may be NULL) skips frames whose entry is 0: none of their outputs is written.
+ * The kernel reads exactly the pixels the refinement's last evaluation read at that pose, so it is valid on a full
+ * pyramid, and on a region-of-interest pyramid (agt_build_pyramid_roi) or after agt_refine_fused for every refinement
+ * that reported left_roi = 0.  Asynchronous on the context's stream, one launch, graph-capturable. */
+int agt_pose_covariance(agt_ctx* ctx, const agt_pyramid* pyr, const double* d_init, const double* d_pose, int n_hyp,
+                        const uint8_t* d_mask, double* d_cov, double* d_info, float* d_sigma2, int32_t* d_n_valid,
+                        uint8_t* d_ok, int batch);
 /* Multi-hypothesis selection: best[b] = argmin_h 2*cost/n_valid (ties -> lowest
  * h); d_best_pose[batch][6] may be NULL. */
 int agt_select_best(agt_ctx* ctx, const double* d_pose, const float* d_cost, const int32_t* d_n_valid,
@@ -362,6 +381,11 @@ int64_t agt_last_h2d_bytes(const agt_ctx* ctx);
 int agt_refine_host(agt_ctx* ctx, const uint8_t* h_frames, int w, int h, int levels, int batch,
                     const double* h_init, int n_hyp, double* h_pose, float* h_cost, int32_t* h_n_valid,
                     int32_t* h_evals, uint8_t* h_status, int32_t* h_best);
+/* agt_pose_covariance from HOST frames [batch][h][w]: uploads the whole frames, builds their pyramids and evaluates
+ * h_init / h_pose [batch][n_hyp][6]; outputs as agt_pose_covariance (h_info, h_sigma2, h_n_valid may be NULL). */
+int agt_pose_covariance_host(agt_ctx* ctx, const uint8_t* h_frames, int w, int h, int levels, int batch, const double* h_init,
+                             const double* h_pose, int n_hyp, double* h_cov, double* h_info, float* h_sigma2,
+                             int32_t* h_n_valid, uint8_t* h_ok);
 
 #ifdef __cplusplus
 }
